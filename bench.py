@@ -5,8 +5,11 @@ penalties {1e2,1e3,1e4,1e5,1e6} = 5,120 independent problems per GPU.
 
   python bench.py --gpus N --steps K --warmup W          our arm (CUDA, through the C ABI)
   python bench.py --impl reference ...                   the reference's CPU solver on the host cores
+  python bench.py ... --dump-outputs DIR                 also write the value path's results as DIR/*.npy
+                                                         (our arm; the reference arm accepts and ignores it)
 
-A "step" is one solve of the whole batch.
+A "step" is one solve of the whole batch; --steps sets the number of timed steps of the value, e2e and
+e2e_plan_api paths (the in-run cpu_baseline sample is one step, the RLE figure the best of four uploads).
   value   K steps of psd_plan_solve (DP + backtrack kernels; the rows are already resident in HBM when the
           timed region starts, as the bench contract asks; no H2D/D2H inside), CUDA events, max over ranks.
   e2e     the DROP-IN path, per step: psd_fpop_disk_batch on the batch's bedGraph FILES (tmpfs) -> text
@@ -15,6 +18,9 @@ A "step" is one solve of the whole batch.
   e2e_plan_api (secondary)  psd_plan_run on host arrays: H2D -> DP -> backtrack -> D2H, no text.
 After the timed steps the result files of 30 problems of the batch are compared with the committed
 reference fixture (tests/golden/golden_fullsize.json, section c2): loss line and sha256(segments).
+The inputs are generated from fixed seeds, so two builds run with the same arguments solve the same
+problems and their --dump-outputs files can be compared array for array.  Nothing is written into the
+source tree (no bytecode either): scratch files go to tmpfs or the temporary directory.
 Multi-GPU: one process per GPU (torchrun), each rank owns its own 5,120 problems (weak scaling, no
 data-path collective); value = all ranks' rows x penalties / max-over-ranks time.
 """
@@ -30,6 +36,7 @@ import sys
 import tempfile
 import time
 
+sys.dont_write_bytecode = True      # the tree may be read-only and must stay as the build left it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 METRIC = "fpop_bedgraph_rows_x_penalties_per_sec"
 UNIT = "rows*penalties/s"
@@ -199,6 +206,35 @@ def check_against_golden(vectors, file_of):
     return n, bad
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(plan, n_rows, out_dir):
+    """What a caller of the timed path (psd_plan_solve, then psd_plan_download) receives, as float64 arrays:
+      loss.npy      [n_probs, 10]  the _loss.tsv fields of every problem (plan.LOSS_COLUMNS), problem order
+      segments.npy  [n_segs, 5]    problem id, chromStart, chromEnd, is_peak, mean: all segments of the
+                                   problems a fixed seeded permutation reaches first while their row counts
+                                   (a bound on the segment counts) fit in 64 MB in all, rows sorted by
+                                   problem id.  The sample depends on the inputs only, never on the results."""
+    import numpy as np
+    n_probs = len(n_rows)
+    os.makedirs(out_dir, exist_ok=True)
+    loss = np.array([list(plan.loss_row(i).values()) for i in range(n_probs)], np.float64)
+    budget = DUMP_BYTES - loss.nbytes - 2 * 4096         # .npy headers
+    picked, used = [], 0
+    for pid in np.random.default_rng(0).permutation(n_probs).tolist():
+        nbytes = 5 * 8 * n_rows[pid]
+        if used + nbytes > budget:
+            break
+        picked.append(pid)
+        used += nbytes
+    parts = [np.column_stack((np.full(len(seg[0]), pid),) + seg).astype(np.float64)
+             for pid in sorted(picked) for seg in [plan.segments(pid)]]
+    np.save(os.path.join(out_dir, "loss.npy"), loss)
+    np.save(os.path.join(out_dir, "segments.npy"), np.concatenate(parts) if parts else np.zeros((0, 5)))
+    return {"dir": out_dir, "problems": n_probs, "problems_with_segments": len(picked)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -209,7 +245,11 @@ def main():
     ap.add_argument("--quick", action="store_true", help="small problems (development only; not a bench value)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-seconds", type=float, default=30.0, help="reference arm: CPU work per step, seconds per core")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the last step's results of the value path as DIR/*.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     config = make_config(args)
@@ -219,6 +259,8 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
+        if args.dump_outputs:
+            print("bench.py: --dump-outputs applies to our arm; the reference arm writes no arrays", file=sys.stderr)
         vectors = build_vectors(0, args.vectors, args.quick)
         td = tempfile.mkdtemp(prefix="psd_ref_", dir=tmp_root)
         try:
@@ -286,6 +328,10 @@ def main():
     plan.upload(stream)
     ms_total, clocks, ms_mine = timed(lambda: plan.solve(stream), args.warmup, args.steps, True)
     st = plan.stats()
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        plan.download(stream)          # outside the timed region: the results of its last step
+        dumped = dump_outputs(plan, [len(p[2]) for p in probs], args.dump_outputs)
     ms_per_step = ms_total / args.steps
     _, total_rows = shard.reduce_time_and_rows(0.0, rows_per_step, dgroup, "cuda")
     value = total_rows / (ms_per_step / 1e3)
@@ -296,7 +342,8 @@ def main():
         dist.all_gather(gathered, t)
         per_rank_ms = [float(g.item()) for g in gathered]
     # ---- secondary: the plan API end to end (host arrays -> H2D -> solve -> D2H) ---------------------------
-    ms_plan, _, _ = timed(lambda: plan.run(stream), 1 if args.warmup > 0 else 0, 1, False)
+    ms_plan, _, _ = timed(lambda: plan.run(stream), 1 if args.warmup > 0 else 0, args.steps, False)
+    ms_plan /= args.steps
     st_plan = plan.stats()
     bad = [i for i in range(len(probs)) if plan.result(i).status != 0]
     if bad:
@@ -413,6 +460,8 @@ def main():
         finally:
             shutil.rmtree(td, ignore_errors=True)
         line["cpu_baseline"] = {"value": ref.rows / secs, "unit": UNIT, "cores": ref.n_threads, "kind": ref.kind, "sample": ref.sample, "seconds": secs}
+    if dumped:
+        line["dump_outputs"] = dumped
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

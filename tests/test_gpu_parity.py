@@ -506,9 +506,21 @@ def test_store_contents_equal_the_reference_db(psd, tmp_path):
     functions -- piece count, max_log_mean, data_i, prev_log_mean of every piece, bit for bit --
     is read back from the GPU store (psd_plan_store_function) and compared."""
     import subprocess
-    from peaksegdisk_b200 import synth
     if not os.path.exists(oracle_bind.REF_BIN):
         pytest.skip("oracle/_ref/ref_fpop not built")
+    _store_equals_db(psd, tmp_path, lambda bg, pen: subprocess.call([oracle_bind.REF_BIN, bg, pen, bg + ".db"], stdout=subprocess.DEVNULL))
+
+
+def test_store_contents_equal_the_oracle_db(psd, tmp_path):
+    """The same comparison against the db the parity oracle writes (oracle/fpop_oracle.cpp, psd_math
+    mode: the reference's DiskVector format, which its size matches in tests/golden), so that the store
+    is checked function by function on every machine, also where the compiled reference is absent."""
+    _store_equals_db(psd, tmp_path, lambda bg, pen: oracle_bind.oracle_disk(bg, pen, bg + ".db", 1))
+
+
+def _store_equals_db(psd, tmp_path, write_db):
+    """write_db(bedgraph, penalty_str) solves the file and leaves bedgraph + '.db'; returns the status."""
+    from peaksegdisk_b200 import synth
     _, ms, me, mc = synth.read_bedgraph(os.path.join(GOLD, "Mono27ac_coverage.bedGraph"))
     probs = [(ms, me, mc, "10.5"), synth.poisson_problem(11, 3000) + ("250",), synth.increasing_problem(150) + ("1000",)]
     plan = psd.Plan(0)
@@ -517,7 +529,7 @@ def test_store_contents_equal_the_reference_db(psd, tmp_path):
     for k, (pid, (s, e, c, pen)) in enumerate(zip(ids, probs)):
         bg = str(tmp_path / ("p%d.bedGraph" % k))
         synth.write_bedgraph(bg, s, e, c)
-        assert subprocess.call([oracle_bind.REF_BIN, bg, pen, bg + ".db"], stdout=subprocess.DEVNULL) == 0
+        assert write_db(bg, pen) == 0
         ref = parse_reference_db(bg + ".db", len(c))
         assert len(ref) == 2 * len(c) - 1 and (0, 0) not in ref      # up_0 does not exist
         n_pieces = 0
