@@ -13,9 +13,7 @@ struct DpKernelParams {
   const DpProblem* problems;
   const int* order;           // problem ids, longest first
   int n_order;
-  int* queue;                 // atomic cursor into order (one per block when bins != null)
-  const int* bins;            // null: one global queue.  Else {begin, end} into order per block: each block works
-                              // through its own share, longest first, and stops refilling when the share is empty
+  int* queue;                 // atomic cursor into order
   DpResult* results;
   StorePool pool;
   int cap_s, ccap_s;          // shared-memory tier (cap_s = 0: disabled, warps start in the global tier)
@@ -28,5 +26,5 @@ struct DpKernelParams {
 
 // fpop_lat.cu: the latency kernel.  Block b solves problem order[b] (no queue).
 int psd_lat_set_smem(size_t smem_bytes);                                   // cudaFuncSetAttribute; returns a cudaError_t
-int psd_lat_max_blocks_per_sm(size_t smem_bytes, int helpers);             // occupancy query
+int psd_lat_resident_blocks(size_t smem_bytes, int helpers);               // occupancy query: blocks per SM
 int psd_lat_launch(const DpKernelParams& P, int grid, size_t smem_bytes, void* stream);   // returns a cudaError_t

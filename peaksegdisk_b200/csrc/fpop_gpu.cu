@@ -34,9 +34,7 @@
 #include "rle_gpu.cuh"
 #include "plan_internal.h"
 
-#ifndef PSD_MAX_WARPS_PER_BLOCK
 #define PSD_MAX_WARPS_PER_BLOCK 16   /* __launch_bounds__(512): 128 registers per thread (fewer registers only add spills; 14-16 warps fit shared memory) */
-#endif
 #define PSD_BT_WARPS_PER_BLOCK 4
 
 #if defined(PSD_TIMING)
@@ -50,13 +48,8 @@ static inline unsigned long long psd_ws_bytes(int cap, int ccap) { return cap > 
 // Two builds of the same kernel: <16,1> one phase-locked block per SM at 128 registers (the default:
 // lowest per-row latency), <14,2> two blocks per SM at 72 registers (28 warps/SM: +18 % on batches of
 // many short problems, -25 % when a long problem sets the critical path; see choose_config()).
-#if defined(PSD_MAXNREG)   // experiment: 14 warps x 32 x 144 registers fill the register file of an SM exactly
-#define PSD_DP_KERNEL_ATTR __maxnreg__(MINB == 1 ? PSD_MAXNREG : 72)
-#else
-#define PSD_DP_KERNEL_ATTR __launch_bounds__(MAXW * 32, MINB)
-#endif
 template <int MAXW, int MINB>
-__global__ void PSD_DP_KERNEL_ATTR
+__global__ void __launch_bounds__(MAXW * 32, MINB)
 fpop_dp_kernel(const DpKernelParams P) {
   uint64_t* etab = (uint64_t*)psd_smem;     // psd_smem: the block's dynamic shared memory (fpop_warp.cuh)
   uint64_t* ltab = etab + 256;
@@ -72,11 +65,6 @@ fpop_dp_kernel(const DpKernelParams P) {
   DpQueue Q;
   Q.problems = P.problems; Q.order = P.order; Q.n_order = P.n_order; Q.cursor = P.queue; Q.results = P.results;
   Q.first_slot = warp * (int)gridDim.x + (int)blockIdx.x;
-  if (P.bins) {
-    Q.first_slot = P.bins[2 * blockIdx.x] + warp;
-    Q.n_order = P.bins[2 * blockIdx.x + 1];
-    Q.cursor = P.queue + blockIdx.x;
-  }
   dp_run_queue(ws_s, ws_g, Q, P.pool);
 #if defined(PSD_TIMING)
   if (threadIdx.x == 0 && blockIdx.x < 160) {   // when did this block run out of work? (ns since kernel start is derived on the host)
@@ -133,7 +121,7 @@ fpop_backtrack_kernel(const BtKernelParams P) {
 namespace {
 thread_local std::string g_last_error;
 std::mutex g_opt_mutex;
-struct Options { int piece_cap = 48; int overflow_cap = 8192; double store_gb = 0; int chunk_kb = 64; int max_warps_per_sm = 0; int blocks_per_sm = 1; int spill_cap = 512; double host_spill_gb = -1; int occupancy_mode = 0; int devices = 1; int queue_mode = 0; int latency_mode = 0; int latency_max_blocks = 16; int spill_mode = 0; double ring_gb = 0; } g_opt;
+struct Options { int piece_cap = 48; int overflow_cap = 8192; double store_gb = 0; int chunk_kb = 64; int spill_cap = 512; double host_spill_gb = -1; int occupancy_mode = 0; int devices = 1; int latency_mode = 0; int latency_max_blocks = 16; int spill_mode = 0; double ring_gb = 0; } g_opt;
 
 bool cuda_ok(cudaError_t e, const char* what) {
   if (e == cudaSuccess) return true;
@@ -156,12 +144,9 @@ int psd_set_option_impl(const char* name, double value) {
   else if (n == "overflow_cap") g_opt.overflow_cap = (int)value;
   else if (n == "store_gb") g_opt.store_gb = value;
   else if (n == "chunk_kb") g_opt.chunk_kb = (int)value;
-  else if (n == "max_warps_per_sm") g_opt.max_warps_per_sm = (int)value;
-  else if (n == "blocks_per_sm") g_opt.blocks_per_sm = std::max(1, (int)value);
   else if (n == "spill_cap") g_opt.spill_cap = std::max(0, (int)value);
   else if (n == "host_spill_gb") g_opt.host_spill_gb = value;
   else if (n == "occupancy_mode") g_opt.occupancy_mode = (int)value;   // 0 auto, 1 one block/SM, 2 two blocks/SM
-  else if (n == "queue_mode") g_opt.queue_mode = (int)value;           // experiment: 0 one global queue, 1 one share of the batch per block
   else if (n == "latency_mode") g_opt.latency_mode = (int)value;       // 0 auto (small waves), 1 always the latency kernel, 2 never
   else if (n == "latency_max_blocks") g_opt.latency_max_blocks = std::max(1, (int)value);   // auto: waves of up to this many problems per SM
   else if (n == "spill_mode") g_opt.spill_mode = (int)value;           // 0 DMA drain of an HBM ring (cudaMemcpyAsync on a side stream), 1 zero-copy stores
@@ -184,7 +169,7 @@ struct psd_plan {
   DpProblem* d_problems = nullptr;
   DpResult* d_results = nullptr;
   int* d_order = nullptr;
-  int* d_queue = nullptr; int* d_bins = nullptr; size_t d_queue_cap = 0;
+  int* d_queue = nullptr;                      // the atomic cursor of the throughput kernel's problem queue
   unsigned long long* d_cursors = nullptr;     // [0] store chunk cursor, [1] segment cursor
   unsigned long long* d_seg_scratch_off = nullptr;
   int *d_scratch_row = nullptr, *d_seg_row = nullptr;
@@ -233,7 +218,7 @@ struct psd_plan {
   ~psd_plan() { release(); }
   void release_device() {
     dfree(d_weight); dfree(d_cov); dfree(d_index); dfree(d_problems); dfree(d_results); dfree(d_order);
-    dfree(d_queue); dfree(d_bins); d_queue_cap = 0; dfree(d_cursors); dfree(d_seg_scratch_off); dfree(d_scratch_row); dfree(d_seg_row);
+    dfree(d_queue); dfree(d_cursors); dfree(d_seg_scratch_off); dfree(d_scratch_row); dfree(d_seg_row);
     dfree(d_scratch_x); dfree(d_seg_x); dfree(d_pool); dfree(d_gws); dfree(d_ring); ring_slots = 0;
     dfree(d_raw); dfree(d_end); dfree(d_end_off); dfree(d_rle_vecs); dfree(d_tile_vec); dfree(d_tile_state); dfree(d_rle_nrows);
     d_raw_cap = d_end_cap = d_rle_vec_cap = d_tile_cap = 0;
@@ -270,12 +255,9 @@ static Options current_options() {
   // environment overrides (tuning experiments)
   if (const char* e = getenv("PSD_PIECE_CAP")) o.piece_cap = atoi(e);
   if (const char* e = getenv("PSD_STORE_GB")) o.store_gb = atof(e);
-  if (const char* e = getenv("PSD_MAX_WARPS")) o.max_warps_per_sm = atoi(e);
-  if (const char* e = getenv("PSD_BLOCKS_PER_SM")) o.blocks_per_sm = std::max(1, atoi(e));
   if (const char* e = getenv("PSD_SPILL_CAP")) o.spill_cap = std::max(0, atoi(e));
   if (const char* e = getenv("PSD_HOST_SPILL_GB")) o.host_spill_gb = atof(e);
   if (const char* e = getenv("PSD_OCCUPANCY_MODE")) o.occupancy_mode = atoi(e);
-  if (const char* e = getenv("PSD_QUEUE_MODE")) o.queue_mode = atoi(e);
   if (const char* e = getenv("PSD_SPILL_MODE")) o.spill_mode = atoi(e);
   if (const char* e = getenv("PSD_LATENCY_MODE")) o.latency_mode = atoi(e);
   if (const char* e = getenv("PSD_LATENCY_MAX_BLOCKS")) o.latency_max_blocks = std::max(1, atoi(e));
@@ -284,8 +266,7 @@ static Options current_options() {
 
 static bool same_options(const Options& a, const Options& b) {
   return a.piece_cap == b.piece_cap && a.overflow_cap == b.overflow_cap && a.store_gb == b.store_gb && a.chunk_kb == b.chunk_kb &&
-         a.max_warps_per_sm == b.max_warps_per_sm && a.blocks_per_sm == b.blocks_per_sm && a.spill_cap == b.spill_cap &&
-         a.host_spill_gb == b.host_spill_gb && a.occupancy_mode == b.occupancy_mode && a.queue_mode == b.queue_mode &&
+         a.spill_cap == b.spill_cap && a.host_spill_gb == b.host_spill_gb && a.occupancy_mode == b.occupancy_mode &&
          a.latency_mode == b.latency_mode && a.latency_max_blocks == b.latency_max_blocks && a.spill_mode == b.spill_mode && a.ring_gb == b.ring_gb;
 }
 
@@ -523,7 +504,7 @@ int psd_plan_upload_impl(psd_plan* p, void* stream_v) {
   // (the pinned staging of the segments is sized at download, from the number of segments found:
   // pinning the worst case of one segment per row cost more than the whole D2H copy)
   if (!p->p_cursors) CK(cudaMallocHost(&p->p_cursors, sizeof(unsigned long long) * 8));
-  if (!p->p_queue_init) CK(cudaMallocHost(&p->p_queue_init, sizeof(int) * 3 * 1024));   // cursors + bins of up to 1024 blocks
+  if (!p->p_queue_init) CK(cudaMallocHost(&p->p_queue_init, sizeof(int)));   // initial value of the queue cursor
   tr.mark("upload: pinned result staging");
   // store pool: sized from free memory unless the option pins it
   size_t free_b = 0, total_b = 0;
@@ -620,7 +601,7 @@ int psd_plan_upload_impl(psd_plan* p, void* stream_v) {
 }
 
 template <int MAXW, int MINB>
-static int configure_one(psd_plan* p, psd_plan::LaunchCfg& L, int cap0, int blocks) {
+static int configure_one(psd_plan* p, psd_plan::LaunchCfg& L, int cap0) {
   int cap = cap0;
   if (cap < 8) cap = 8;
   cap = (cap + 3) & ~3;   // multiples of 4 keep every list array 16-byte aligned (bulk copies of the record store)
@@ -628,16 +609,15 @@ static int configure_one(psd_plan* p, psd_plan::LaunchCfg& L, int cap0, int bloc
     const int ccap = 2 * cap;
     const size_t per_warp = psd_ws_bytes(cap, ccap);
     // each block also costs ~1 KB of reserved shared memory
-    int w = (int)((((size_t)p->prop.sharedMemPerMultiprocessor / blocks) - 1024 - PSD_TAB_BYTES) / per_warp);
+    int w = (int)((((size_t)p->prop.sharedMemPerMultiprocessor / MINB) - 1024 - PSD_TAB_BYTES) / per_warp);
     w = std::min(w, (int)(((size_t)p->prop.sharedMemPerBlockOptin - PSD_TAB_BYTES) / per_warp));
     w = std::min(w, MAXW);
-    if (p->opt.max_warps_per_sm > 0) w = std::min(w, std::max(1, p->opt.max_warps_per_sm / blocks));
     for (; w >= 1; w--) {   // registers may allow fewer warps than shared memory does
       const size_t smem = PSD_TAB_BYTES + (size_t)w * per_warp;
       CK(cudaFuncSetAttribute(fpop_dp_kernel<MAXW, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       int nb = 0;
       CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fpop_dp_kernel<MAXW, MINB>, w * 32, smem));
-      if (nb >= blocks) { L.ok = true; L.blocks = blocks; L.wpb = w; L.cap = cap; L.ccap = ccap; L.smem = smem; return 0; }
+      if (nb >= MINB) { L.ok = true; L.blocks = MINB; L.wpb = w; L.cap = cap; L.ccap = ccap; L.smem = smem; return 0; }
     }
     cap = ((cap / 2) + 3) & ~3;
     if (cap < 8) { L.ok = false; return 0; }
@@ -646,10 +626,10 @@ static int configure_one(psd_plan* p, psd_plan::LaunchCfg& L, int cap0, int bloc
 
 static int configure_kernel(psd_plan* p) {
   if (p->configured) return 0;
-  int rc = configure_one<PSD_MAX_WARPS_PER_BLOCK, 1>(p, p->cfg[0], p->opt.piece_cap, p->opt.blocks_per_sm);
+  int rc = configure_one<PSD_MAX_WARPS_PER_BLOCK, 1>(p, p->cfg[0], p->opt.piece_cap);
   if (rc) return rc;
   if (!p->cfg[0].ok) { g_last_error = "cannot fit the DP kernel's shared memory"; return PSD_ERR_CUDA; }
-  rc = configure_one<14, 2>(p, p->cfg[1], p->opt.piece_cap / 2, 2);
+  rc = configure_one<14, 2>(p, p->cfg[1], p->opt.piece_cap / 2);
   if (rc) return rc;
   p->configured = true;
   return 0;
@@ -967,7 +947,7 @@ int psd_plan_solve_impl(psd_plan* p, void* stream_v) {
       grid = n;
       // helper warps pay with one block per SM (-9 % per row); with more resident blocks they cost more than they give (measured)
       K.lat_help = per_sm <= 1 ? 1 : 0;
-      S.piece_cap = K.cap_s; S.warps_per_sm = (K.lat_help ? 4 : PSD_LAT_WARPS) * std::min(per_sm, std::max(1, psd_lat_max_blocks_per_sm(smem, K.lat_help)));
+      S.piece_cap = K.cap_s; S.warps_per_sm = (K.lat_help ? 4 : PSD_LAT_WARPS) * std::min(per_sm, std::max(1, psd_lat_resident_blocks(smem, K.lat_help)));
     } else if (!global_tier) {
       // shared-memory tier, with a per-warp global workspace the kernel moves to (and back from)
       // when a row's functions outgrow shared memory
@@ -992,43 +972,10 @@ int psd_plan_solve_impl(psd_plan* p, void* stream_v) {
       K.gws = p->d_gws;
     }
     tr.mark("solve: descriptors + workspace");
-    if ((size_t)grid > p->d_queue_cap || !p->d_queue) {
-      dfree(p->d_queue); dfree(p->d_bins); p->d_queue_cap = 0;
-      const size_t qn = std::max(4, grid);
-      CK(cudaMalloc(&p->d_queue, sizeof(int) * qn));
-      CK(cudaMalloc(&p->d_bins, sizeof(int) * 2 * qn));
-      p->d_queue_cap = qn;
-    }
-    K.bins = nullptr;
-    std::vector<int> binned;
-    if (!lat && !global_tier && p->opt.queue_mode == 1 && grid <= 1024 && n > grid * wpb) {
-      // EXPERIMENT (profiles/README.md): one share of the wave per block, longest-first onto the
-      // least loaded block by rows.  A block that has emptied its share does not refill, so the warps
-      // still working on long problems get the SM to themselves.
-      std::vector<std::vector<int>> bin(grid);
-      std::priority_queue<std::pair<double, int>, std::vector<std::pair<double, int>>, std::greater<std::pair<double, int>>> load;
-      for (int b = 0; b < grid; b++) load.push({0.0, b});
-      for (int g : todo) {
-        auto top = load.top(); load.pop();
-        bin[top.second].push_back(g);
-        load.push({top.first + (double)p->probs[p->gpu_ids[g]].n_rows, top.second});
-      }
-      binned.reserve(n);
-      for (int b = 0; b < grid; b++) {
-        p->p_queue_init[1024 + 2 * b] = (int)binned.size();
-        binned.insert(binned.end(), bin[b].begin(), bin[b].end());
-        p->p_queue_init[1024 + 2 * b + 1] = (int)binned.size();
-        p->p_queue_init[b] = p->p_queue_init[1024 + 2 * b] + wpb;   // the first wpb of a share are taken statically
-      }
-      CK(cudaMemcpyAsync(p->d_order, binned.data(), sizeof(int) * n, cudaMemcpyHostToDevice, st));
-      CK(cudaMemcpyAsync(p->d_queue, p->p_queue_init, sizeof(int) * grid, cudaMemcpyHostToDevice, st));
-      CK(cudaMemcpyAsync(p->d_bins, p->p_queue_init + 1024, sizeof(int) * 2 * grid, cudaMemcpyHostToDevice, st));
-      K.bins = p->d_bins;
-    } else {
-      CK(cudaMemcpyAsync(p->d_order, todo.data(), sizeof(int) * n, cudaMemcpyHostToDevice, st));
-      p->p_queue_init[0] = grid * wpb;   // slots below this are assigned statically
-      CK(cudaMemcpyAsync(p->d_queue, p->p_queue_init, sizeof(int), cudaMemcpyHostToDevice, st));
-    }
+    if (!p->d_queue) CK(cudaMalloc(&p->d_queue, sizeof(int)));
+    CK(cudaMemcpyAsync(p->d_order, todo.data(), sizeof(int) * n, cudaMemcpyHostToDevice, st));
+    *p->p_queue_init = grid * wpb;   // slots below this are assigned statically
+    CK(cudaMemcpyAsync(p->d_queue, p->p_queue_init, sizeof(int), cudaMemcpyHostToDevice, st));
     K.queue = p->d_queue;
     CK(cudaMemsetAsync(p->d_cursors, 0, sizeof(unsigned long long), st));   // recycle the store pool
     CK(cudaMemsetAsync(p->d_cursors + 2, 0, sizeof(unsigned long long), st));

@@ -49,7 +49,7 @@ int psd_lat_set_smem(size_t smem_bytes) {
   return (int)cudaFuncSetAttribute(fpop_dp_lat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
 }
 
-int psd_lat_max_blocks_per_sm(size_t smem_bytes, int helpers) {
+int psd_lat_resident_blocks(size_t smem_bytes, int helpers) {
   int nb = 0;
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fpop_dp_lat_kernel, helpers ? PSD_LAT_THREADS : PSD_LAT_WARPS * 32, smem_bytes) != cudaSuccess) return 0;
   return nb;

@@ -41,10 +41,9 @@
 // This header is compiled by nvcc for the product and, unmodified, by g++ against
 // tests/emu/warp_emu.h (PSD_EMU) where fibers stand in for the lanes of one or several warps -- a test
 // tool only.
-// Experiment switches (never set in the product build): PSD_TIMING (cycle counters), PSD_SPEC,
-// PSD_RETURN_NUM/DEN, PSD_INLINE_MATH / PSD_INLINE_EXP / PSD_INLINE_LOG, PSD_NOINLINE_ROOTS,
-// PSD_NOINLINE_OPS, PSD_NO_SHARED_HINT, PSD_NO_BULK_STORE;
-// what they showed is in profiles/README.md.
+// Builds: PSD_G32 the latency kernel (above); PSD_TIMING the cycle-counter build (`make timing`, read
+// by tools/prof_timing*.py, prof_tail.py, prof_newton_rounds.py); PSD_EMU the emulator, PSD_EMU_STATS
+// its operator-size histograms (tools/emu_stats.py).
 #pragma once
 #include "psd_math.h"
 
@@ -144,25 +143,10 @@ extern unsigned long long psd_emu_stats[8][65];
 #else
 #define PSD_STAT(slot, leader, v) do {} while (0)
 #endif
-// While a flat stretch is open the pieces ahead are tested speculatively, PSD_SPEC lanes per round
 #if defined(PSD_G32)
 #define PSD_G 32             /* lanes per operator group: a whole warp (latency kernel) */
 #else
 #define PSD_G 16             /* lanes per operator group (half a warp) */
-#endif
-#ifndef PSD_SPEC
-#define PSD_SPEC PSD_G
-#endif
-// a problem running from its global workspace returns to shared memory when both functions have at
-// most PSD_RETURN_NUM/PSD_RETURN_DEN of the shared-memory capacity
-#ifndef PSD_RETURN_NUM
-#define PSD_RETURN_NUM 1
-#define PSD_RETURN_DEN 2
-#endif
-#if defined(PSD_NO_BULK_STORE)   /* experiment switch: records written by the lanes even from shared memory */
-#define PSD_BULK_STORE false
-#else
-#define PSD_BULK_STORE true
 #endif
 #define PSD_EPS 1e-12        /* NEWTON_EPSILON, src/funPieceListLog.cpp:9 */
 #define PSD_MAX_STEPS 100    /* NEWTON_STEPS,   src/funPieceListLog.cpp:10 */
@@ -181,7 +165,7 @@ extern unsigned long long psd_emu_stats[8][65];
 struct PList { double* base; int n; };
 // Shared-memory tier: the operators are instantiated a second time with the promise that every list
 // and scratch pointer is a shared-memory address (32-bit LDS/STS instead of generic 64-bit LD/ST).
-#if defined(PSD_EMU) || defined(PSD_NO_SHARED_HINT)
+#if defined(PSD_EMU)
 #define PSD_ASSUME_SHARED(p) do {} while (0)
 #else
 #define PSD_ASSUME_SHARED(p) __builtin_assume(__isShared((const void*)(p)))
@@ -226,21 +210,8 @@ extern __shared__ __align__(16) unsigned char psd_smem[];
 #define PSD_ETAB ((const uint64_t*)psd_smem)
 #define PSD_LTAB (((const uint64_t*)psd_smem) + 256)
 #endif
-#if defined(PSD_INLINE_MATH)
-PSD_DEV double w_exp(double x) { return psd_exp(x, PSD_ETAB); }
-PSD_DEV double w_log(double x) { return psd_log(x, PSD_LTAB); }
-#else
-#if defined(PSD_INLINE_EXP)
-PSD_DEV double w_exp(double x) { return psd_exp(x, PSD_ETAB); }
-#else
 PSD_DEVNI double w_exp(double x) { return psd_exp(x, PSD_ETAB); }
-#endif
-#if defined(PSD_INLINE_LOG)
-PSD_DEV double w_log(double x) { return psd_log(x, PSD_LTAB); }
-#else
 PSD_DEVNI double w_log(double x) { return psd_log(x, PSD_LTAB); }
-#endif
-#endif
 
 // rescale applied while writing an operator's output:  ((v * mul) + add) * inv  per coefficient,
 // i.e. multiply(W_{t-1}); add(w, -z*w, 0); multiply(1/W_t)   (src/PeakSegFPOPLog.cpp:316-321)
@@ -269,25 +240,15 @@ PSD_DEV double pc_abs(double v) { return v < 0 ? -v : v; }
 // The two big operators are inlined into the kernel body, each at its single call site per tier
 // (the executed footprint per phase is unchanged, argument passing through local memory and 320 B of
 // spills go away: +1-2 %).  Real functions mattered only before the phase lock, when the warps of
-// an SM were at unrelated program counters.  -DPSD_NOINLINE_OPS restores them; exp/log stay real
-// functions (inlining those loses 3-4 %: they have ~20 call sites).
-#if defined(PSD_NOINLINE_OPS)
-#define PSD_OP PSD_DEVNI
-#else
-#define PSD_OP PSD_DEV
-#endif
+// an SM were at unrelated program counters.  exp/log stay real functions (w_exp / w_log above;
+// inlining those loses 3-4 %: they have ~20 call sites).
 // The two Newton solvers are inlined into their three call sites (the code per phase stays the same
 // size, the 8-double argument shuffle of a call disappears: +4 % on config 2, +6 % on short
-// problems, profiles/README.md).  -DPSD_NOINLINE_ROOTS keeps them as real functions.
-#if defined(PSD_NOINLINE_ROOTS)
-#define PSD_ROOT PSD_DEVNI
-#else
-#define PSD_ROOT PSD_DEV
-#endif
+// problems, profiles/README.md).
 // get_smaller_root (:129-190): Newton in log space from argmin-1.
 // x0 = argmin, c0 = cost(x0), cl = cost(lo) are passed in (the reference recomputes the same values).
-PSD_ROOT double root_left(double a, double b, double c, double lo, double level,
-                           double x0, double c0, double cl) {
+PSD_DEV double root_left(double a, double b, double c, double lo, double level,
+                          double x0, double c0, double cl) {
   if ((level < cl && cl < c0) || (level > cl && cl > c0)) return lo - 1;
   double x = x0 - 1;
   double f, pos_f = PSD_INF, pos_x = PSD_INF, neg_f = -PSD_INF, neg_x = PSD_INF;
@@ -313,8 +274,8 @@ PSD_ROOT double root_left(double a, double b, double c, double lo, double level,
 
 // get_larger_root (:69-127): Newton in mean space from argmin_mean+1; returns log(root).
 // m0 = argmin_mean, c0 = PoissonLoss(m0), cr = cost(hi) are passed in.
-PSD_ROOT double root_right(double a, double b, double c, double hi, double level,
-                            double m0, double c0, double cr) {
+PSD_DEV double root_right(double a, double b, double c, double hi, double level,
+                           double m0, double c0, double cr) {
   if ((c0 < cr && cr < level) || (c0 > cr && cr > level)) return hi + 1;
   double m = m0 + 1;
   double f, pos_f = PSD_INF, pos_m = PSD_INF, neg_f = -PSD_INF, neg_m = PSD_INF;
@@ -369,7 +330,7 @@ PSD_DEV void pl_emit(const WarpWs ws, const PList out, int k, double a, double b
 //   * less stamps back_i, adds the penalty to c and +0.0 to a and b (add(0,0,c), :618-625); more only stamps
 // Output pieces are produced in scan order and, for dir 1, reversed at the end.
 template <bool SH>
-PSD_OP int min_mono_op(const WarpWs ws, const PList in, const PList out, double dmin, int stamp, double cshift, int dir) {
+PSD_DEV int min_mono_op(const WarpWs ws, const PList in, const PList out, double dmin, int stamp, double cshift, int dir) {
   if (SH) { PSD_ASSUME_SHARED(in.base); PSD_ASSUME_SHARED(out.base); PSD_ASSUME_SHARED(ws.scratch); PSD_ASSUME_SHARED(ws.flags); }
   const int lane = psd_glane();   // lane within this 16-lane group
   const int cap = ws.cap;
@@ -458,7 +419,7 @@ PSD_OP int min_mono_op(const WarpWs ws, const PList in, const PList out, double 
         stat_windows++;
         int flag = 0;
         double r = PSD_INF;   // no root: fails the interval test below
-        if (valid && u >= pos && u < pos + PSD_SPEC) {
+        if (valid && u >= pos && u < pos + PSD_G) {
           if (b == 0) {
             if (dir) r = w_log((level - c) / a);
             else if (a < 0) flag = 3;   // the reference throws here ("should never happen")
@@ -471,7 +432,7 @@ PSD_OP int min_mono_op(const WarpWs ws, const PList in, const PList out, double 
           }
         }
         const unsigned mask = psd_g_ballot(flag != 0);
-        if (!mask) { pos = (pos + PSD_SPEC < end) ? pos + PSD_SPEC : end; continue; }   // still flat: next window
+        if (!mask) { pos = (pos + PSD_G < end) ? pos + PSD_G : end; continue; }   // still flat: next window
         const int src = psd_ffs(mask) - 1;
         const int fl = psd_g_shfl_i(flag, src);
         const double r_s = psd_g_shfl_d(r, src), eout_s = psd_g_shfl_d(eout, src);
@@ -842,8 +803,8 @@ PSD_DEV void lat_helper_loop(LatHelp* H, int g) {
 // same two lists of the OTHER chain (the call is converged over both half-warps and stage 2 pools
 // the intervals of both chains over all 32 lanes).
 template <bool SH>
-PSD_OP int min_env_op(const WarpWs ws, const PList f, const PList g, const PList of, const PList og, const PList out,
-                      double dmin, const Rescale rs) {
+PSD_DEV int min_env_op(const WarpWs ws, const PList f, const PList g, const PList of, const PList og, const PList out,
+                       double dmin, const Rescale rs) {
   if (SH) {
     PSD_ASSUME_SHARED(f.base); PSD_ASSUME_SHARED(g.base); PSD_ASSUME_SHARED(of.base); PSD_ASSUME_SHARED(og.base);
     PSD_ASSUME_SHARED(out.base); PSD_ASSUME_SHARED(ws.scratch); PSD_ASSUME_SHARED(ws.flags);
@@ -1443,6 +1404,12 @@ PSD_DEV void pl_move(const double* src, int scap, double* dst, int dcap, int n) 
   }
 }
 
+// A problem running from its global workspace (in_g) returns to shared memory (capacity cap_s,
+// 0 = disabled) once both functions fill at most half of it.
+PSD_DEV bool back_to_shared(bool in_g, int n_up, int n_down, int cap_s) {
+  return in_g && cap_s > 0 && 2 * n_up <= cap_s && 2 * n_down <= cap_s;
+}
+
 #if !defined(PSD_G32)
 // order[] lists problem ids longest first.  Slot q = warp_in_block * n_blocks + block is taken
 // statically by that warp (so the longest problems land one per SM and a small batch spreads over
@@ -1611,7 +1578,7 @@ PSD_DEV void dp_run_queue(const WarpWs& ws_s, const WarpWs& ws_g, const DpQueue&
           if (off == ~0ull) status = PSD_ST_STORE_EXHAUSTED;
           else {
             // bulk copies need a device-memory destination: HBM, or the writer's ring slot
-            const bool dev_dst = PSD_BULK_STORE && (sw.slot >= 0 || off < sp.n_chunks * sp.chunk_bytes);
+            const bool dev_dst = sw.slot >= 0 || off < sp.n_chunks * sp.chunk_bytes;
             if (in_g) store_write<false>(ws, store_wptr(sp, sw, off), t, upP, downP, false);
             else store_write<true>(ws, store_wptr(sp, sw, off), t, upP, downP, dev_dst);
             if (lane == (t & 31)) my_off = off;
@@ -1633,7 +1600,7 @@ PSD_DEV void dp_run_queue(const WarpWs& ws_s, const WarpWs& ws_g, const DpQueue&
             res->pad_ = n_spill;
           }
           fetch = true;
-        } else if (in_g && ws_s.cap > 0 && PSD_RETURN_DEN * upP.n <= PSD_RETURN_NUM * ws_s.cap && PSD_RETURN_DEN * downP.n <= PSD_RETURN_NUM * ws_s.cap) {
+        } else if (back_to_shared(in_g, upP.n, downP.n, ws_s.cap)) {
           // both functions fit comfortably again: move back to shared memory
           psd_syncwarp();
           pl_move(upP.base, ws_g.cap, ws_list(ws_s, 0), ws_s.cap, upP.n);
@@ -1819,7 +1786,7 @@ PSD_DEV void dp_run_latency(const WarpWs& ws_s, const WarpWs& ws_g, const DpProb
       const unsigned long long off = store_alloc_cta(sp, sw, store_record_bytes(upP.n, downP.n), sh, grp);
       if (off == ~0ull) status = PSD_ST_STORE_EXHAUSTED;
       else {
-        const bool dev_dst = PSD_BULK_STORE && (sw.slot >= 0 || off < sp.n_chunks * sp.chunk_bytes);
+        const bool dev_dst = sw.slot >= 0 || off < sp.n_chunks * sp.chunk_bytes;
         if (in_g) store_write_fn<false>(ws, store_wptr(sp, sw, off), t, grp ? downP : upP, grp, upP.n, downP.n, false);
         else store_write_fn<true>(ws, store_wptr(sp, sw, off), t, grp ? downP : upP, grp, upP.n, downP.n, dev_dst);
         if (grp == 0) {
@@ -1845,7 +1812,7 @@ PSD_DEV void dp_run_latency(const WarpWs& ws_s, const WarpWs& ws_g, const DpProb
       }
       break;
     }
-    if (in_g && ws_s.cap > 0 && PSD_RETURN_DEN * upP.n <= PSD_RETURN_NUM * ws_s.cap && PSD_RETURN_DEN * downP.n <= PSD_RETURN_NUM * ws_s.cap) {
+    if (back_to_shared(in_g, upP.n, downP.n, ws_s.cap)) {
       // both functions fit comfortably again: move back to shared memory
       if (grp == 0) pl_move(upP.base, ws_g.cap, ws_list(ws_s, 0), ws_s.cap, upP.n);
       else pl_move(downP.base, ws_g.cap, ws_list(ws_s, 1), ws_s.cap, downP.n);

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Same-box A/B of kernel build variants (run it inside ONE gpurun call: GPUs of the pool differ by ~10 %).
-#   tools/ab_variants.sh build "-DPSD_DEFER_NEWTON" "-DPSD_NOINLINE_OPS" ...   # here: cross-compile one .so per flag set
+#   tools/ab_variants.sh build "-DSOME_FLAG" "-DSOME_FLAG -DOTHER_FLAG" ...    # here: cross-compile one .so per flag set
 #   gpurun -- 'tools/ab_variants.sh run'                                       # on the GPU box: parity + timings per variant
 # Variant 0 is always the product build (no extra flags).
 set -e

@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Experiment: config-2 vectors at ONE penalty (function sizes differ a lot between penalties) under
-the launch configuration / queue mode given in the environment (PSD_OCCUPANCY_MODE, PSD_QUEUE_MODE).
+the launch configuration given in the environment (PSD_OCCUPANCY_MODE).
 usage: python tools/prof_shares.py <penalty> [n_vectors=1024] [copies=5]"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -19,6 +19,6 @@ for rep in range(2):
 plan.download()
 mi = sum(plan.loss_row(i)["mean.intervals"] for i in range(0, len(plan), 37)) / len(range(0, len(plan), 37))
 mx = max(plan.loss_row(i)["max.intervals"] for i in range(len(plan)))
-print("penalty=%g occupancy=%s queue=%s: dp_ms=%.1f rows/s=%.3e warps/sm=%d mean.intervals=%.2f max.intervals=%d overflow_tier_problems=%d" % (
-    pen, os.environ.get("PSD_OCCUPANCY_MODE", "0"), os.environ.get("PSD_QUEUE_MODE", "0"), st["dp_ms"], rows / st["dp_ms"] * 1e3,
+print("penalty=%g occupancy=%s: dp_ms=%.1f rows/s=%.3e warps/sm=%d mean.intervals=%.2f max.intervals=%d overflow_tier_problems=%d" % (
+    pen, os.environ.get("PSD_OCCUPANCY_MODE", "0"), st["dp_ms"], rows / st["dp_ms"] * 1e3,
     st["warps_per_sm"], mi, mx, st["n_overflow_tier"]), flush=True)
