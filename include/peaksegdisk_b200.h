@@ -154,6 +154,38 @@ int psd_last_batch_stats(psd_batch_stats *out);
 int psd_write_bedgraph(const char *path, const char *chrom, int64_t n_rows, const int32_t *chromStart,
                        const int32_t *chromEnd, const int32_t *count);
 
+/* ---- coverage from aligned reads --------------------------------------------------------------
+ * One problem is the reads of one region of one sample.  The coverage of base b is the number of
+ * reads with start <= b < end (bedtools genomecov -bga, clipped to the region); the rows are the
+ * maximal runs of equal coverage, zero runs included, and tile [region_start, region_end) exactly, so
+ * they are valid psd_plan_add / psd_write_bedgraph input.  Reads partly outside the region are
+ * clipped, reads wholly outside are ignored; a region without reads gives one zero row. */
+typedef struct psd_reads {
+  int64_t n_reads;
+  const int32_t *read_start, *read_end;    /* half-open [start, end), any order */
+  int32_t region_start, region_end;        /* rows tile [region_start, region_end) */
+} psd_reads;
+typedef struct psd_coverage psd_coverage;  /* rows of every problem, on the host */
+typedef struct psd_coverage_stats {
+  double device_ms;                        /* CUDA events around H2D + zero-fill + scatter + scan + RLE + D2H, summed over waves */
+  double kernel_ms;                        /* zero-fill + scatter + scan + RLE only */
+  int64_t reads, bases, rows, h2d_bytes, d2h_bytes;   /* reads and bases of the problems that went to the device */
+  int32_t n_problems, n_waves;
+} psd_coverage_stats;
+/* Computes the rows of n_problems problems on the device, in waves whose dense per-base buffers fit
+ * the "coverage_gb" budget (psd_set_option).  Inputs are checked on the host before any device work:
+ * start < 0, end <= start, region_start < 0, region_end <= region_start, a region longer than
+ * 0x3fffffff bases, a null read array with n_reads > 0 and n_reads outside [0, 2^31) return PSD_ERR_ARG
+ * and psd_last_error() names the problem and read.  device < 0: the current device.  Returns 0 and
+ * *out (free it with psd_coverage_free), or PSD_ERR_ARG / PSD_ERR_CUDA and no handle. */
+int psd_coverage_from_reads(int device, int n_problems, const psd_reads *problems, psd_coverage **out);
+/* Rows of problem i (-1 if i is out of range). */
+int64_t psd_coverage_n_rows(const psd_coverage *cov, int i);
+/* Copies problem i's rows; the arrays need psd_coverage_n_rows(cov, i) entries. */
+int psd_coverage_rows(const psd_coverage *cov, int i, int32_t *chromStart, int32_t *chromEnd, int32_t *count);
+int psd_coverage_get_stats(const psd_coverage *cov, psd_coverage_stats *out);
+void psd_coverage_free(psd_coverage *cov);
+
 /* Inspection of the cost-function store (replaces DiskVector::read, src/PeakSegFPOPLog.cpp:103-117,
  * for tests and tools): the stored function `which` (0 = up, 1 = down) of bedGraph row `row` of
  * problem id, in the reference's record fields (src/PeakSegFPOPLog.cpp:18-34: max_log_mean, data_i,
@@ -174,7 +206,9 @@ int psd_plan_store_function(psd_plan *plan, int id, int row, int which, int cap,
  * the latency kernel -- one problem per block, one chain per warp -- for few or long problems, never beyond
  * "latency_max_blocks" (16) problems per SM; 1 = always the latency kernel; 2 = never),
  * "devices" (GPUs one psd_fpop_disk_batch call may use: 1 = the current device (default), k = the
- * first k, <= 0 = all; problems are dealt longest-first, one plan and host thread per GPU). */
+ * first k, <= 0 = all; problems are dealt longest-first, one plan and host thread per GPU),
+ * "coverage_gb" (device budget of one psd_coverage_from_reads wave: dense per-base buffer, rows and
+ * reads; 0 = automatic, half of the free HBM; a problem larger than the budget runs in a wave of its own). */
 int psd_set_option(const char *name, double value);
 
 int psd_device_count(void);

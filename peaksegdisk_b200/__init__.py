@@ -5,10 +5,10 @@ Plan (plan.py).  All solves run in libpeaksegdisk_b200.so; importing fails if it
 """
 from . import _lib
 from .api import (PeakSegFPOP_file, PeakSegFPOP_file_batch, PeakSegFPOP_dir, PeakSegFPOP_df, PeakSegFPOP_vec,
-                  PeakSegFPOP_vec_batch,
+                  PeakSegFPOP_vec_batch, coverage_from_reads,
                   sequentialSearch_dir, sequentialSearch_batch, writeBedGraph, col_name_list, r_paste)
-from .plan import Plan, solve_batch, solve_counts_batch
+from .plan import Plan, solve_batch, solve_counts_batch, solve_reads_batch
 
 __all__ = ["PeakSegFPOP_file", "PeakSegFPOP_file_batch", "PeakSegFPOP_dir", "PeakSegFPOP_df", "PeakSegFPOP_vec", "PeakSegFPOP_vec_batch",
            "sequentialSearch_dir", "sequentialSearch_batch", "writeBedGraph", "col_name_list", "r_paste", "Plan", "solve_batch",
-           "solve_counts_batch"]
+           "solve_counts_batch", "coverage_from_reads", "solve_reads_batch"]

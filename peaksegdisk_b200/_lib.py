@@ -37,12 +37,24 @@ class PsdBatchStats(C.Structure):
                 ("n_devices", C.c_int32), ("n_launches", C.c_int32), ("n_waves", C.c_int32), ("n_latency_waves", C.c_int32)]
 
 
+class PsdReads(C.Structure):
+    _fields_ = [("n_reads", C.c_int64), ("read_start", C.POINTER(C.c_int32)), ("read_end", C.POINTER(C.c_int32)),
+                ("region_start", C.c_int32), ("region_end", C.c_int32)]
+
+
+class PsdCoverageStats(C.Structure):
+    _fields_ = [("device_ms", C.c_double), ("kernel_ms", C.c_double), ("reads", C.c_int64), ("bases", C.c_int64),
+                ("rows", C.c_int64), ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64), ("n_problems", C.c_int32),
+                ("n_waves", C.c_int32)]
+
+
 # every symbol include/peaksegdisk_b200.h declares (tests check the library exports all of them)
 C_ABI_SYMBOLS = [
     "psd_fpop_disk", "psd_fpop_disk_batch", "psd_status_message", "psd_last_error", "psd_plan_create",
     "psd_plan_destroy", "psd_plan_add", "psd_plan_add_counts", "psd_plan_size", "psd_plan_upload", "psd_plan_solve", "psd_plan_download",
     "psd_plan_run", "psd_plan_result", "psd_plan_segments", "psd_plan_get_stats", "psd_plan_set_penalty", "psd_plan_store_function", "psd_write_bedgraph", "psd_last_batch_stats",
     "psd_set_option", "psd_device_count", "psd_release_cache",
+    "psd_coverage_from_reads", "psd_coverage_n_rows", "psd_coverage_rows", "psd_coverage_get_stats", "psd_coverage_free",
     "_Z16PeakSegFPOP_diskPcS_S_",   # the reference's own C++-linkage entry (src/PeakSegFPOPLog.h:15)
 ]
 
@@ -95,6 +107,16 @@ def _load():
     lib.psd_set_option.restype = C.c_int
     lib.psd_set_option.argtypes = [C.c_char_p, C.c_double]
     lib.psd_device_count.restype = C.c_int
+    lib.psd_coverage_from_reads.restype = C.c_int
+    lib.psd_coverage_from_reads.argtypes = [C.c_int, C.c_int, C.POINTER(PsdReads), C.POINTER(C.c_void_p)]
+    lib.psd_coverage_n_rows.restype = C.c_int64
+    lib.psd_coverage_n_rows.argtypes = [C.c_void_p, C.c_int]
+    lib.psd_coverage_rows.restype = C.c_int
+    lib.psd_coverage_rows.argtypes = [C.c_void_p, C.c_int, i32p, i32p, i32p]
+    lib.psd_coverage_get_stats.restype = C.c_int
+    lib.psd_coverage_get_stats.argtypes = [C.c_void_p, C.POINTER(PsdCoverageStats)]
+    lib.psd_coverage_free.restype = None
+    lib.psd_coverage_free.argtypes = [C.c_void_p]
     return lib
 
 

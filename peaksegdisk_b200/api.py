@@ -263,6 +263,54 @@ def PeakSegFPOP_vec_batch(count_vecs, pen_nums):
     return out
 
 
+def coverage_from_reads(reads, region=None, device=-1):
+    """Coverage of aligned reads as a bedGraph data.frame, computed on the device (not an R function of
+    the reference: its Spatial_correlation vignette builds coverage from reads in R before solving).
+
+    reads: data.frame with columns chrom, chromStart, chromEnd (half-open read intervals, any order;
+    other columns are ignored).  region: None (each chromosome's [min chromStart, max chromEnd)) or a
+    dict chrom -> (start, end); reads are clipped to their region and reads outside it are ignored, and
+    a dict chromosome without reads gives one zero row.  All chromosomes go to the device in one call.
+    Returns a data.frame with col_name_list["coverage"] columns, chromosomes in order of first appearance
+    (then the dict's other chromosomes), whose rows tile each region: input for writeBedGraph /
+    PeakSegFPOP_df / sequentialSearch_dir."""
+    from .plan import coverage_rows
+    if not isinstance(reads, pd.DataFrame):
+        raise ValueError("reads must be data.frame")
+    if not all(c in reads.columns for c in ("chrom", "chromStart", "chromEnd")):
+        raise ValueError("reads must have columns chrom, chromStart, chromEnd")
+    for col in ("chromStart", "chromEnd"):
+        if len(reads) and not pd.api.types.is_integer_dtype(reads[col]):
+            raise ValueError("reads$%s must be integer" % col)
+    if region is not None and not isinstance(region, dict):
+        raise ValueError("region must be None or a dict chrom -> (start, end)")
+    region = region or {}
+    chroms = list(pd.unique(reads["chrom"]))
+    seen = set(chroms)
+    chroms += [c for c in region if c not in seen]
+    groups = reads.groupby("chrom", sort=False).indices if len(reads) else {}
+    starts, ends = reads["chromStart"].to_numpy(), reads["chromEnd"].to_numpy()
+    problems = []
+    for ch in chroms:
+        idx = groups.get(ch, np.zeros(0, np.int64))
+        s, e = starts[idx], ends[idx]
+        if ch in region:
+            if len(region[ch]) != 2:
+                raise ValueError("region[%r] must be (start, end)" % (ch,))
+            a, b = region[ch]
+        else:
+            a, b = s.min(), e.max()
+        problems.append((s, e, a, b))
+    rows, _ = coverage_rows(problems, device)
+    n = [len(r[2]) for r in rows]
+    if not rows:
+        return pd.DataFrame({k: pd.Series(dtype=object if k == "chrom" else np.int32) for k in col_name_list["coverage"]})
+    return pd.DataFrame({"chrom": np.repeat(np.array(chroms, dtype=object), n),
+                         "chromStart": np.concatenate([r[0] for r in rows]),
+                         "chromEnd": np.concatenate([r[1] for r in rows]),
+                         "count": np.concatenate([r[2] for r in rows])})
+
+
 def _solve_many(requests):
     """requests: list of (problem_dir, penalty_str).  Everything that is not already cached goes to
     the GPU in ONE batched launch; returns the PeakSegFPOP_dir result of every request."""

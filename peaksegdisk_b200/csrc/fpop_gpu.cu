@@ -3,6 +3,9 @@
 // Launch structure (one CUDA stream, no host sync between kernels):
 //   rle_encode_kernel      (upload, count-vector problems only) run-length encodes raw count vectors
 //                          into the DP's rows (rle_gpu.cuh).
+//   reads_scatter_kernel, coverage_scan_kernel, then rle_encode_kernel
+//                          (psd_coverage_from_reads only, not part of a plan) per-base coverage of
+//                          aligned reads and its rows (coverage_gpu.cuh).
 //   fpop_dp_kernel<W,B>    persistent warps; each warp takes problems (longest first) from an atomic
 //                          queue and runs dp_run_queue() (fpop_warp.cuh): the whole DP of one
 //                          (bedGraph x penalty), piece lists in shared memory (moving to a per-warp
@@ -32,6 +35,7 @@
 #include <vector>
 #include "dp_params.h"
 #include "rle_gpu.cuh"
+#include "coverage_gpu.cuh"
 #include "plan_internal.h"
 
 #define PSD_MAX_WARPS_PER_BLOCK 16   /* __launch_bounds__(512): 128 registers per thread (fewer registers only add spills; 14-16 warps fit shared memory) */
@@ -121,7 +125,7 @@ fpop_backtrack_kernel(const BtKernelParams P) {
 namespace {
 thread_local std::string g_last_error;
 std::mutex g_opt_mutex;
-struct Options { int piece_cap = 48; int overflow_cap = 8192; double store_gb = 0; int chunk_kb = 64; int spill_cap = 512; double host_spill_gb = -1; int occupancy_mode = 0; int devices = 1; int latency_mode = 0; int latency_max_blocks = 16; int spill_mode = 0; double ring_gb = 0; } g_opt;
+struct Options { int piece_cap = 48; int overflow_cap = 8192; double store_gb = 0; int chunk_kb = 64; int spill_cap = 512; double host_spill_gb = -1; int occupancy_mode = 0; int devices = 1; int latency_mode = 0; int latency_max_blocks = 16; int spill_mode = 0; double ring_gb = 0; double coverage_gb = 0; } g_opt;
 
 bool cuda_ok(cudaError_t e, const char* what) {
   if (e == cudaSuccess) return true;
@@ -152,6 +156,7 @@ int psd_set_option_impl(const char* name, double value) {
   else if (n == "spill_mode") g_opt.spill_mode = (int)value;           // 0 DMA drain of an HBM ring (cudaMemcpyAsync on a side stream), 1 zero-copy stores
   else if (n == "ring_gb") g_opt.ring_gb = value;                      // HBM ring of the DMA drain (0 = automatic)
   else if (n == "devices") g_opt.devices = (int)value;                 // 1 current device only, k first k GPUs, <= 0 all
+  else if (n == "coverage_gb") g_opt.coverage_gb = value;              // psd_coverage_from_reads wave budget (0 = half of free HBM)
   else return PSD_ERR_ARG;
   return 0;
 }
@@ -1190,6 +1195,265 @@ int psd_plan_store_function_impl(psd_plan* p, int id, int row, int which, int ca
   CK(fetch(hi, off + R.hi[which], 8ull * n));
   CK(fetch(back_x, off + R.bx[which], 8ull * n));
   CK(fetch(back_i, off + R.bi[which], 4ull * n));
+  return 0;
+}
+
+// ---- coverage from aligned reads (psd_coverage_from_reads, coverage_gpu.cuh) -------------------------
+namespace {
+// Device arena, pinned staging and events of one psd_coverage_from_reads call, freed on every return.
+struct CovScratch {
+  unsigned char* d_arena = nullptr; size_t arena_bytes = 0;
+  int32_t *p_start = nullptr, *p_end = nullptr; size_t p_reads_cap = 0;   // reads of a wave
+  int32_t *p_cov = nullptr, *p_rend = nullptr; size_t p_rows_cap = 0;     // rows of a wave
+  int* p_small = nullptr;                                                 // n_rows of a wave's problems + 2 error flags
+  cudaEvent_t ev[6]; bool ev_ok = false;
+  ~CovScratch() {
+    if (d_arena) cudaFree(d_arena);
+    if (p_start) cudaFreeHost(p_start); if (p_end) cudaFreeHost(p_end);
+    if (p_cov) cudaFreeHost(p_cov); if (p_rend) cudaFreeHost(p_rend); if (p_small) cudaFreeHost(p_small);
+    if (ev_ok) for (auto& e : ev) cudaEventDestroy(e);
+  }
+};
+
+struct CovJob {
+  int prob;
+  int64_t n_reads, n_bases, row_bound, n_tiles;
+};
+
+inline size_t cov_align(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// device bytes of a wave (the arena is carved in this order, see psd_coverage_from_reads_impl)
+size_t cov_wave_bytes(int64_t n_probs, int64_t bases, int64_t rows, int64_t reads, int64_t tiles) {
+  return cov_align(4 * bases) + 2 * cov_align(4 * reads) + 3 * cov_align(4 * rows) + cov_align(sizeof(RleVec) * n_probs) +
+         cov_align(8 * (n_probs + 1)) + 2 * cov_align(4 * n_probs) + cov_align(4 * tiles) + 2 * cov_align(8 * (tiles + 1));
+}
+}  // namespace
+
+// Host checks (before any device work), then waves of problems whose device footprint fits the
+// "coverage_gb" budget: H2D of the reads, zero-fill, scatter, scan, RLE, D2H of the rows.  Problems
+// without a read inside their region never reach the device: their one zero row is made here.
+int psd_coverage_from_reads_impl(int device, int n, const psd_reads* P, psd_coverage** out) {
+  if (!out) { g_last_error = "psd_coverage_from_reads: out is null"; return PSD_ERR_ARG; }
+  *out = nullptr;
+  if (n < 0 || (n > 0 && !P)) { g_last_error = "psd_coverage_from_reads: n_problems < 0 or problems is null"; return PSD_ERR_ARG; }
+  std::vector<int64_t> inside(n, 0);   // reads that overlap the region
+  std::vector<std::string> err(n);
+  auto check = [&](int k) {
+    const psd_reads& q = P[k];
+    char msg[192];
+    if (q.n_reads < 0 || q.n_reads >= (1ll << 31)) snprintf(msg, sizeof msg, "n_reads %lld is outside [0, 2^31)", (long long)q.n_reads);
+    else if (q.n_reads > 0 && (!q.read_start || !q.read_end)) snprintf(msg, sizeof msg, "read_start or read_end is null with n_reads %lld", (long long)q.n_reads);
+    else if (q.region_start < 0) snprintf(msg, sizeof msg, "region_start %d < 0", q.region_start);
+    else if (q.region_end <= q.region_start) snprintf(msg, sizeof msg, "region_end %d <= region_start %d", q.region_end, q.region_start);
+    else if ((int64_t)q.region_end - q.region_start > 0x3fffffff) snprintf(msg, sizeof msg, "region of %lld bases is longer than 0x3fffffff", (long long)q.region_end - q.region_start);
+    else {
+      int64_t m = 0;
+      for (int64_t r = 0; r < q.n_reads; r++) {
+        const int32_t s = q.read_start[r], e = q.read_end[r];
+        if (s < 0) { snprintf(msg, sizeof msg, "read %lld: start %d < 0", (long long)r, s); err[k] = msg; return; }
+        if (e <= s) { snprintf(msg, sizeof msg, "read %lld: end %d <= start %d", (long long)r, e, s); err[k] = msg; return; }
+        m += (e > q.region_start && s < q.region_end);
+      }
+      inside[k] = m;
+      return;
+    }
+    err[k] = msg;
+  };
+  int64_t all_reads = 0;
+  for (int k = 0; k < n; k++) all_reads += P[k].n_reads > 0 ? P[k].n_reads : 0;
+  if (all_reads > (1 << 22)) parallel_for(n, check);
+  else for (int k = 0; k < n; k++) check(k);
+  for (int k = 0; k < n; k++)
+    if (!err[k].empty()) { g_last_error = "psd_coverage_from_reads: problem " + std::to_string(k) + ": " + err[k]; return PSD_ERR_ARG; }
+
+  std::unique_ptr<psd_coverage> C(new psd_coverage());
+  psd_coverage_stats& S = C->stats;
+  memset(&S, 0, sizeof S);
+  S.n_problems = n;
+  C->row_off.assign(1, 0);
+  auto emit = [&](int32_t s, int32_t e, int32_t c) { C->chrom_start.push_back(s); C->chrom_end.push_back(e); C->count.push_back(c); };
+  int next_emit = 0;
+  auto emit_empty_until = [&](int k_end) {   // problems before k_end that have no read in their region: one zero row
+    for (; next_emit < k_end; next_emit++) {
+      emit(P[next_emit].region_start, P[next_emit].region_end, 0);
+      C->row_off.push_back((int64_t)C->count.size());
+    }
+  };
+  std::vector<CovJob> jobs;
+  for (int k = 0; k < n; k++) {
+    if (!inside[k]) continue;
+    const int64_t nb = (int64_t)P[k].region_end - P[k].region_start;
+    jobs.push_back({k, P[k].n_reads, nb, std::min(nb, 2 * inside[k] + 1), (nb + PSD_RLE_TILE - 1) / PSD_RLE_TILE});
+  }
+  if (!jobs.empty()) {
+    int ndev = 0;
+    if (!cuda_ok(cudaGetDeviceCount(&ndev), "cudaGetDeviceCount")) return PSD_ERR_CUDA;
+    if (ndev == 0) { g_last_error = "no CUDA device"; return PSD_ERR_CUDA; }
+    if (device < 0) CK(cudaGetDevice(&device));
+    CK(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    CK(cudaGetDeviceProperties(&prop, device));
+    if (prop.major < 10) { g_last_error = "peaksegdisk_b200 is built for sm_100a only"; return PSD_ERR_CUDA; }
+    CovScratch X;
+    for (auto& e : X.ev) CK(cudaEventCreate(&e));
+    X.ev_ok = true;
+    // waves: consecutive jobs while their footprint fits the budget (a job larger than it runs alone)
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    const double gb = current_options().coverage_gb;
+    const size_t budget = gb > 0 ? (size_t)(gb * (double)(1ull << 30)) : free_b / 2;
+    std::vector<std::pair<size_t, size_t>> waves;   // [first job, end job)
+    size_t arena = 0, max_reads = 0;
+    for (size_t j0 = 0; j0 < jobs.size();) {
+      size_t j1 = j0;
+      int64_t bases = 0, rows = 0, reads = 0, tiles = 0;
+      size_t bytes = 0;
+      for (; j1 < jobs.size(); j1++) {
+        const CovJob& J = jobs[j1];
+        const size_t b = cov_wave_bytes((int64_t)(j1 - j0 + 1), bases + J.n_bases, rows + J.row_bound, reads + J.n_reads, tiles + J.n_tiles);
+        if (j1 > j0 && b > budget) break;
+        bases += J.n_bases; rows += J.row_bound; reads += J.n_reads; tiles += J.n_tiles; bytes = b;
+      }
+      waves.push_back({j0, j1});
+      arena = std::max(arena, bytes); max_reads = std::max(max_reads, (size_t)reads);
+      j0 = j1;
+    }
+    CK(cudaMalloc(&X.d_arena, arena));
+    X.arena_bytes = arena;
+    CK(cudaMallocHost(&X.p_start, 4 * max_reads));
+    CK(cudaMallocHost(&X.p_end, 4 * max_reads));
+    X.p_reads_cap = max_reads;
+    size_t max_probs = 0;
+    for (const auto& w : waves) max_probs = std::max(max_probs, w.second - w.first);
+    CK(cudaMallocHost(&X.p_small, sizeof(int) * (max_probs + 2)));
+    const cudaStream_t st = 0;
+    for (const auto& w : waves) {
+      const int np = (int)(w.second - w.first);
+      std::vector<RleVec> vecs(np);
+      std::vector<long long> read_off(np + 1, 0);
+      std::vector<int> region(np), tile_vec;
+      int64_t bases = 0, rows = 0, reads = 0;
+      for (int j = 0; j < np; j++) {
+        const CovJob& J = jobs[w.first + j];
+        RleVec& v = vecs[j];
+        v.raw_off = bases; v.row_off = rows; v.n_pos = (int)J.n_bases; v.tile0 = (int)tile_vec.size();
+        tile_vec.insert(tile_vec.end(), (size_t)J.n_tiles, j);
+        region[j] = P[J.prob].region_start;
+        read_off[j] = reads;
+        bases += J.n_bases; rows += J.row_bound; reads += J.n_reads;
+      }
+      read_off[np] = reads;
+      const int n_tiles = (int)tile_vec.size();
+      auto stage = [&](int j) {
+        const psd_reads& q = P[jobs[w.first + j].prob];
+        memcpy(X.p_start + read_off[j], q.read_start, 4 * (size_t)q.n_reads);
+        memcpy(X.p_end + read_off[j], q.read_end, 4 * (size_t)q.n_reads);
+      };
+      if (reads > (1 << 22)) parallel_for(np, stage);
+      else for (int j = 0; j < np; j++) stage(j);
+      // carve the arena (the order cov_wave_bytes() counts)
+      unsigned char* a = X.d_arena;
+      auto carve = [&](size_t b) { unsigned char* r = a; a += cov_align(b); return r; };
+      int* d_cov = (int*)carve(4 * bases);
+      int* d_start = (int*)carve(4 * reads);
+      int* d_end = (int*)carve(4 * reads);
+      int* d_rcov = (int*)carve(4 * rows);
+      int* d_rend = (int*)carve(4 * rows);
+      int* d_rw = (int*)carve(4 * rows);
+      RleVec* d_vecs = (RleVec*)carve(sizeof(RleVec) * np);
+      long long* d_read_off = (long long*)carve(8 * (np + 1));
+      int* d_region = (int*)carve(4 * np);
+      int* d_nrows = (int*)carve(4 * np);
+      int* d_tile_vec = (int*)carve(4 * n_tiles);
+      unsigned long long* d_scan_state = (unsigned long long*)carve(8 * (n_tiles + 1));   // look-back words, then ticket and error flag
+      unsigned long long* d_rle_state = (unsigned long long*)carve(8 * (n_tiles + 1));
+      CK(cudaEventRecord(X.ev[0], st));
+      CK(cudaMemcpyAsync(d_start, X.p_start, 4 * reads, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(d_end, X.p_end, 4 * reads, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(d_vecs, vecs.data(), sizeof(RleVec) * np, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(d_read_off, read_off.data(), 8 * (np + 1), cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(d_region, region.data(), 4 * np, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(d_tile_vec, tile_vec.data(), 4 * (size_t)n_tiles, cudaMemcpyHostToDevice, st));
+      CK(cudaEventRecord(X.ev[1], st));
+      CK(cudaMemsetAsync(d_cov, 0, 4 * bases, st));
+      CK(cudaMemsetAsync(d_scan_state, 0, 8 * (n_tiles + 1), st));
+      CK(cudaMemsetAsync(d_rle_state, 0, 8 * (n_tiles + 1), st));
+      CovScatterParams A;
+      A.read_start = d_start; A.read_end = d_end; A.n_reads = reads; A.read_off = d_read_off; A.region_start = d_region;
+      A.vecs = d_vecs; A.n_probs = np; A.delta = d_cov;
+      const long long want_blocks = (reads + 255) / 256;
+      reads_scatter_kernel<<<(int)std::min<long long>(want_blocks, 16ll * prop.multiProcessorCount), 256, 0, st>>>(A);
+      CK(cudaGetLastError());
+      CovScanParams B;
+      B.vecs = d_vecs; B.tile_vec = d_tile_vec; B.n_tiles = n_tiles; B.cov = d_cov;
+      B.tile_state = d_scan_state; B.ticket = (unsigned int*)(d_scan_state + n_tiles); B.error = (int*)(B.ticket + 1);
+      coverage_scan_kernel<<<n_tiles, PSD_RLE_WARPS * 32, 0, st>>>(B);
+      CK(cudaGetLastError());
+      RleParams R;
+      R.vecs = d_vecs; R.tile_vec = d_tile_vec; R.n_tiles = n_tiles; R.n_vecs = np;
+      R.raw = d_cov; R.coverage = d_rcov; R.chrom_end = d_rend; R.weight = d_rw;
+      R.tile_state = d_rle_state; R.n_rows = d_nrows;
+      R.ticket = (unsigned int*)(d_rle_state + n_tiles); R.error = (int*)(R.ticket + 1);
+      rle_encode_kernel<<<n_tiles, PSD_RLE_WARPS * 32, 0, st>>>(R);
+      CK(cudaGetLastError());
+      CK(cudaEventRecord(X.ev[2], st));
+      CK(cudaMemcpyAsync(X.p_small, d_nrows, 4 * np, cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(X.p_small + np, B.error, 4, cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(X.p_small + np + 1, R.error, 4, cudaMemcpyDeviceToHost, st));
+      CK(cudaEventRecord(X.ev[3], st));
+      CK(cudaStreamSynchronize(st));
+      if (X.p_small[np] || X.p_small[np + 1]) { g_last_error = "device coverage: look-back gave up"; return PSD_ERR_INTERNAL; }
+      int64_t got = 0;
+      for (int j = 0; j < np; j++) {
+        const int nr = X.p_small[j];
+        if (nr < 1 || nr > jobs[w.first + j].row_bound) { g_last_error = "device coverage: row count outside its bound"; return PSD_ERR_INTERNAL; }
+        got += nr;
+      }
+      if ((size_t)got > X.p_rows_cap) {
+        if (X.p_cov) cudaFreeHost(X.p_cov); if (X.p_rend) cudaFreeHost(X.p_rend);
+        X.p_cov = X.p_rend = nullptr; X.p_rows_cap = 0;
+        CK(cudaMallocHost(&X.p_cov, 4 * got));
+        CK(cudaMallocHost(&X.p_rend, 4 * got));
+        X.p_rows_cap = got;
+      }
+      // rows: exact counts per problem, packed into the staging
+      CK(cudaEventRecord(X.ev[4], st));
+      int64_t o = 0;
+      for (int j = 0; j < np; j++) {
+        const int nr = X.p_small[j];
+        CK(cudaMemcpyAsync(X.p_cov + o, d_rcov + vecs[j].row_off, 4 * (size_t)nr, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(X.p_rend + o, d_rend + vecs[j].row_off, 4 * (size_t)nr, cudaMemcpyDeviceToHost, st));
+        o += nr;
+      }
+      CK(cudaEventRecord(X.ev[5], st));
+      CK(cudaStreamSynchronize(st));
+      float t01 = 0, t13 = 0, t45 = 0, t12 = 0;
+      cudaEventElapsedTime(&t01, X.ev[0], X.ev[1]); cudaEventElapsedTime(&t13, X.ev[1], X.ev[3]);
+      cudaEventElapsedTime(&t45, X.ev[4], X.ev[5]); cudaEventElapsedTime(&t12, X.ev[1], X.ev[2]);
+      S.device_ms += t01 + t13 + t45; S.kernel_ms += t12;
+      S.reads += reads; S.bases += bases; S.n_waves++;
+      S.h2d_bytes += 8 * reads + (int64_t)(sizeof(RleVec) + 12) * np + 8 + 4 * (int64_t)n_tiles;
+      S.d2h_bytes += 4 * (np + 2) + 8 * got;
+      o = 0;
+      for (int j = 0; j < np; j++) {
+        const int k = jobs[w.first + j].prob;
+        emit_empty_until(k);
+        const int nr = X.p_small[j], r0 = P[k].region_start;
+        int prev = r0;
+        for (int r = 0; r < nr; r++) {
+          const int e = X.p_rend[o + r] + r0;
+          emit(prev, e, X.p_cov[o + r]);
+          prev = e;
+        }
+        o += nr;
+        C->row_off.push_back((int64_t)C->count.size());
+        next_emit = k + 1;
+      }
+    }
+  }
+  emit_empty_until(n);
+  S.rows = (int64_t)C->count.size();
+  *out = C.release();
   return 0;
 }
 

@@ -652,6 +652,33 @@ int psd_last_batch_stats(psd_batch_stats* out) {
   return 0;
 }
 
+int psd_coverage_from_reads(int device, int n_problems, const psd_reads* problems, psd_coverage** out) {
+  return psd_coverage_from_reads_impl(device, n_problems, problems, out);
+}
+
+int64_t psd_coverage_n_rows(const psd_coverage* cov, int i) {
+  if (!cov || i < 0 || i + 1 >= (int64_t)cov->row_off.size()) return -1;
+  return cov->row_off[i + 1] - cov->row_off[i];
+}
+
+int psd_coverage_rows(const psd_coverage* cov, int i, int32_t* chromStart, int32_t* chromEnd, int32_t* count) {
+  const int64_t n = psd_coverage_n_rows(cov, i);
+  if (n < 0 || !chromStart || !chromEnd || !count) return PSD_ERR_ARG;
+  const int64_t o = cov->row_off[i];
+  memcpy(chromStart, cov->chrom_start.data() + o, sizeof(int32_t) * n);
+  memcpy(chromEnd, cov->chrom_end.data() + o, sizeof(int32_t) * n);
+  memcpy(count, cov->count.data() + o, sizeof(int32_t) * n);
+  return 0;
+}
+
+int psd_coverage_get_stats(const psd_coverage* cov, psd_coverage_stats* out) {
+  if (!cov || !out) return PSD_ERR_ARG;
+  *out = cov->stats;
+  return 0;
+}
+
+void psd_coverage_free(psd_coverage* cov) { delete cov; }
+
 int psd_set_option(const char* name, double value) { return name ? psd_set_option_impl(name, value) : PSD_ERR_ARG; }
 int psd_device_count(void) { return psd_device_count_impl(); }
 void psd_release_cache(void) { psd_plan_drop_parked(); }

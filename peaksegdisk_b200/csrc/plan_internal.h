@@ -75,6 +75,14 @@ template <class F> void parallel_for(int n, F fn) {
   for (auto& th : pool) th.join();
 }
 
+// Result of psd_coverage_from_reads: the rows of problem i are [row_off[i], row_off[i + 1]).
+struct psd_coverage {
+  std::vector<int64_t> row_off;
+  std::vector<int32_t> chrom_start, chrom_end, count;
+  psd_coverage_stats stats;
+};
+int psd_coverage_from_reads_impl(int device, int n_problems, const psd_reads* problems, psd_coverage** out);
+
 struct psd_plan;
 psd_plan* psd_plan_create_impl(int device);
 void psd_plan_destroy_impl(psd_plan* p);

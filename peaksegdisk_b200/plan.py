@@ -18,6 +18,22 @@ def _i32(a):
     return a, a.ctypes.data_as(C.POINTER(C.c_int32))
 
 
+def _coords(a, what):
+    """int32 view of a coordinate array; non-integer or out-of-int32 values raise ValueError."""
+    a = np.asarray(a)
+    if a.size and not np.issubdtype(a.dtype, np.integer):
+        raise ValueError("%s must be integer" % what)
+    return _i32(a)
+
+
+def _coord(x, what):
+    if isinstance(x, bool) or not isinstance(x, (int, np.integer)):
+        raise ValueError("%s must be an integer" % what)
+    if not -2147483648 <= int(x) <= 2147483647:
+        raise ValueError("%s does not fit a 32-bit integer" % what)
+    return int(x)
+
+
 class Plan:
     """A batch of independent problems.  add() copies rows to the host side of the plan;
     upload()/solve()/download() are the three timed phases; run() does all three."""
@@ -145,5 +161,53 @@ def solve_counts_batch(problems, device=-1, stream=0):
     vectors at once; the vectors are run-length encoded on the device.  Returns (plan, ids)."""
     plan = Plan(device)
     ids = [plan.add_counts(v, pen) for (v, pen) in problems]
+    plan.run(stream)
+    return plan, ids
+
+
+def coverage_rows(problems, device=-1):
+    """problems: iterable of (read_start, read_end, region_start, region_end), reads half-open and in any
+    order.  The per-base coverage of each region and its run-length encoding into rows, computed on the
+    device in ONE psd_coverage_from_reads call (coverage_gpu.cuh).  Returns (rows, stats): rows[i] is
+    problem i's (chromStart, chromEnd, count) int32 arrays, which tile [region_start, region_end);
+    stats is the call's psd_coverage_stats as a dict."""
+    problems = list(problems)
+    arr = (_lib.PsdReads * max(1, len(problems)))()
+    keep = []   # the int32 copies must outlive the call
+    for i, (rs, re_, a, b) in enumerate(problems):
+        s, sp = _coords(rs, "read_start")
+        e, ep = _coords(re_, "read_end")
+        if len(s) != len(e):
+            raise ValueError("read_start and read_end must have the same length")
+        keep += [s, e]
+        arr[i].n_reads = len(s); arr[i].read_start = sp; arr[i].read_end = ep
+        arr[i].region_start = _coord(a, "region_start"); arr[i].region_end = _coord(b, "region_end")
+    h = C.c_void_p()
+    rc = _lib.lib.psd_coverage_from_reads(int(device), len(problems), arr, C.byref(h))
+    if rc:
+        raise (ValueError if rc == 111 else RuntimeError)("peaksegdisk_b200: " + _lib.status_text(rc))
+    try:
+        rows = []
+        for i in range(len(problems)):
+            n = _lib.lib.psd_coverage_n_rows(h, i)
+            s = np.empty(n, np.int32); e = np.empty(n, np.int32); c = np.empty(n, np.int32)
+            p32 = C.POINTER(C.c_int32)
+            _lib.lib.psd_coverage_rows(h, i, s.ctypes.data_as(p32), e.ctypes.data_as(p32), c.ctypes.data_as(p32))
+            rows.append((s, e, c))
+        st = _lib.PsdCoverageStats()
+        _lib.lib.psd_coverage_get_stats(h, C.byref(st))
+        return rows, {name: getattr(st, name) for name, _ in st._fields_}
+    finally:
+        _lib.lib.psd_coverage_free(h)
+
+
+def solve_reads_batch(problems, device=-1, stream=0):
+    """problems: iterable of (read_start, read_end, region_start, region_end, penalty): aligned reads in,
+    segmentations out.  One coverage call for all problems (coverage_rows), then Plan.add on each
+    problem's rows and one run.  Returns (plan, ids)."""
+    problems = list(problems)
+    rows, _ = coverage_rows([p[:4] for p in problems], device)
+    plan = Plan(device)
+    ids = [plan.add(s, e, c, p[4]) for (s, e, c), p in zip(rows, problems)]
     plan.run(stream)
     return plan, ids

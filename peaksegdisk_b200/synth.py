@@ -69,6 +69,23 @@ def read_bedgraph(path):
     return a[0, 0], a[:, 1].astype(np.int32), a[:, 2].astype(np.int32), a[:, 3].astype(np.int32)
 
 
+def reads(seed, n_reads, length, start=0, n_peaks=None, read_len=(36, 300)):
+    """Seeded aligned reads for [start, start + length): half uniform background, half around n_peaks
+    centres (default one per 20 kb), lengths uniform in read_len.  Returns unsorted half-open int32
+    (read_start, read_end); a read may run past the region's end."""
+    rng = np.random.default_rng(seed)
+    if n_peaks is None:
+        n_peaks = max(1, length // 20000)
+    centres = rng.integers(0, length, size=n_peaks)
+    n_bg = n_reads // 2
+    pos = np.concatenate([rng.integers(0, length, size=n_bg),
+                          centres[rng.integers(0, n_peaks, size=n_reads - n_bg)] + rng.normal(0, 300, size=n_reads - n_bg).astype(np.int64)])
+    pos = np.clip(pos, 0, length - 1) + start
+    rng.shuffle(pos)
+    rl = rng.integers(read_len[0], read_len[1] + 1, size=n_reads)
+    return pos.astype(np.int32), (pos + rl).astype(np.int32)
+
+
 def hg19_problem(chrom_index, sample_index, base_weight, base_count, scale_rows=1.0):
     """One config-4 problem: tile the Mono27ac (weight, count) rows up to the chromosome's row
     target, redraw counts, RLE, re-accumulate coordinates (SURVEY.md 8d, C4)."""
