@@ -134,6 +134,68 @@ int psd_plan_get_stats(const psd_plan *plan, psd_stats *out);
 /* Replaces problem id's penalty (used by the sequential search to re-solve the same rows). */
 int psd_plan_set_penalty(psd_plan *plan, int id, double penalty, int penalty_is_inf);
 
+/* ---- label errors (PeakError semantics, 0-based half-open coordinates) ------------------------
+ * A label [chromStart, chromEnd) of kind 0 noPeaks, 1 peaks, 2 peakStart, 3 peakEnd is scored on the
+ * peak segments [ps, pe) of a problem's segmentation: o = peaks with ps < chromEnd and chromStart < pe,
+ * a = peak starts in [chromStart, chromEnd), b = peak ends in (chromStart, chromEnd].
+ *   noPeaks: fp = o > 0, fn = 0;  peaks: fp = 0, fn = o == 0;  peakStart: fp = a > 1, fn = a == 0;
+ *   peakEnd: fp = b > 1, fn = b == 0.  possible_fp = kind != 1, possible_fn = kind != 0.
+ * Labels are scored on the device right after the backtrack, only for plans that have labels. */
+typedef struct psd_label_errors {
+  int32_t fp, fn, possible_fp, possible_fn, errors;   /* sums over the problem's labels; errors = fp + fn */
+} psd_label_errors;
+/* Copies n labels of problem id (n = 0 removes them).  Each needs chromStart < chromEnd inside the
+ * problem's [first chromStart, last chromEnd) and kind 0..3; they may be unsorted and overlap.  Returns
+ * 0, or PSD_ERR_ARG with the problem and label named in psd_last_error(). */
+int psd_plan_set_labels(psd_plan *plan, int id, int64_t n, const int32_t *chromStart, const int32_t *chromEnd,
+                        const int32_t *kind);
+/* After psd_plan_solve: the totals of problem id and, if the arrays are not null, fp / fn per label in
+ * the order they were set.  Returns 0, the problem's solver status, or PSD_ERR_ARG (no labels, not solved). */
+int psd_plan_label_errors(const psd_plan *plan, int id, psd_label_errors *total, int32_t *fp, int32_t *fn);
+
+/* ---- exact model-selection path (CROPS) ------------------------------------------------------
+ * Every model that is optimal for some penalty in [pen_min, pen_max], found by solving at the crossing
+ * penalty of each pair of neighbouring models (Haynes, Eckley and Fearnhead 2017); every pending pair of
+ * every problem is solved in one batched plan solve per round.  With labels, each model's label errors
+ * are counted on the device and the target interval is the widest (in log penalty) run of consecutive
+ * models with the fewest errors. */
+typedef struct psd_path_problem {
+  int64_t n_rows;                                    /* rows as for psd_plan_add */
+  const int32_t *chromStart, *chromEnd, *coverage;
+  int64_t n_labels;                                  /* labels as for psd_plan_set_labels (0: none) */
+  const int32_t *label_start, *label_end, *label_kind;
+} psd_path_problem;
+typedef struct psd_path_model {
+  double min_lambda, max_lambda;   /* the penalties for which this model is optimal */
+  double penalty;                  /* the penalty of the solve that found it */
+  double total_loss;
+  int32_t peaks, segments;
+  int32_t fp, fn, possible_fp, possible_fn, errors;   /* zero without labels */
+  int32_t pad_;
+} psd_path_model;
+typedef struct psd_path psd_path;
+typedef struct psd_path_stats {
+  double dp_ms, backtrack_ms, label_ms;   /* device time summed over rounds */
+  int64_t rows_solved;                     /* rows x solves of the non-trivial solves */
+  int64_t h2d_bytes, d2h_bytes;
+  int32_t rounds, solves, models, n_problems;
+} psd_path_stats;
+/* Solves the path of n_problems problems on [pen_min, pen_max] (pen_max may be INFINITY).  Inputs are
+ * checked on the host before any device work: NaN or negative pen_min, pen_min > pen_max, an infinite
+ * pen_min with a finite pen_max, n_problems < 0 and bad rows or labels return PSD_ERR_ARG, naming the
+ * problem in psd_last_error().  A problem whose solve fails keeps that status and no models; the others
+ * finish.  device < 0: the current device.  Returns 0 and *out (free with psd_path_free), or an error. */
+int psd_model_path(int device, int n_problems, const psd_path_problem *problems, double pen_min, double pen_max,
+                   psd_path **out);
+int psd_path_status(const psd_path *path, int i);        /* problem i's status (PSD_ERR_ARG if i is out of range) */
+int psd_path_n_models(const psd_path *path, int i);      /* -1 if i is out of range */
+/* Copies problem i's models, sorted by peaks ascending; the array needs psd_path_n_models entries. */
+int psd_path_models(const psd_path *path, int i, psd_path_model *models);
+/* Problem i's target interval: *errors = -1 (and NaN penalties) when it has no labels or no models. */
+int psd_path_target(const psd_path *path, int i, double *min_lambda, double *max_lambda, int32_t *errors);
+int psd_path_get_stats(const psd_path *path, psd_path_stats *out);
+void psd_path_free(psd_path *path);
+
 /* Where the wall time of the process's last psd_fpop_disk / psd_fpop_disk_batch call went. */
 typedef struct psd_batch_stats {
   double parse_ms;           /* bedGraph text -> rows (distinct files on all host cores) + penalty parsing */

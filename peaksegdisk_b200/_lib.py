@@ -48,6 +48,29 @@ class PsdCoverageStats(C.Structure):
                 ("n_waves", C.c_int32)]
 
 
+class PsdLabelErrors(C.Structure):
+    _fields_ = [("fp", C.c_int32), ("fn", C.c_int32), ("possible_fp", C.c_int32), ("possible_fn", C.c_int32),
+                ("errors", C.c_int32)]
+
+
+class PsdPathProblem(C.Structure):
+    _fields_ = [("n_rows", C.c_int64), ("chromStart", C.POINTER(C.c_int32)), ("chromEnd", C.POINTER(C.c_int32)),
+                ("coverage", C.POINTER(C.c_int32)), ("n_labels", C.c_int64), ("label_start", C.POINTER(C.c_int32)),
+                ("label_end", C.POINTER(C.c_int32)), ("label_kind", C.POINTER(C.c_int32))]
+
+
+class PsdPathModel(C.Structure):
+    _fields_ = [("min_lambda", C.c_double), ("max_lambda", C.c_double), ("penalty", C.c_double), ("total_loss", C.c_double),
+                ("peaks", C.c_int32), ("segments", C.c_int32), ("fp", C.c_int32), ("fn", C.c_int32),
+                ("possible_fp", C.c_int32), ("possible_fn", C.c_int32), ("errors", C.c_int32), ("pad_", C.c_int32)]
+
+
+class PsdPathStats(C.Structure):
+    _fields_ = [("dp_ms", C.c_double), ("backtrack_ms", C.c_double), ("label_ms", C.c_double), ("rows_solved", C.c_int64),
+                ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64), ("rounds", C.c_int32), ("solves", C.c_int32),
+                ("models", C.c_int32), ("n_problems", C.c_int32)]
+
+
 # every symbol include/peaksegdisk_b200.h declares (tests check the library exports all of them)
 C_ABI_SYMBOLS = [
     "psd_fpop_disk", "psd_fpop_disk_batch", "psd_status_message", "psd_last_error", "psd_plan_create",
@@ -55,6 +78,8 @@ C_ABI_SYMBOLS = [
     "psd_plan_run", "psd_plan_result", "psd_plan_segments", "psd_plan_get_stats", "psd_plan_set_penalty", "psd_plan_store_function", "psd_write_bedgraph", "psd_last_batch_stats",
     "psd_set_option", "psd_device_count", "psd_release_cache",
     "psd_coverage_from_reads", "psd_coverage_n_rows", "psd_coverage_rows", "psd_coverage_get_stats", "psd_coverage_free",
+    "psd_plan_set_labels", "psd_plan_label_errors", "psd_model_path", "psd_path_status", "psd_path_n_models",
+    "psd_path_models", "psd_path_target", "psd_path_get_stats", "psd_path_free",
     "_Z16PeakSegFPOP_diskPcS_S_",   # the reference's own C++-linkage entry (src/PeakSegFPOPLog.h:15)
 ]
 
@@ -117,6 +142,24 @@ def _load():
     lib.psd_coverage_get_stats.argtypes = [C.c_void_p, C.POINTER(PsdCoverageStats)]
     lib.psd_coverage_free.restype = None
     lib.psd_coverage_free.argtypes = [C.c_void_p]
+    lib.psd_plan_set_labels.restype = C.c_int
+    lib.psd_plan_set_labels.argtypes = [C.c_void_p, C.c_int, C.c_int64, i32p, i32p, i32p]
+    lib.psd_plan_label_errors.restype = C.c_int
+    lib.psd_plan_label_errors.argtypes = [C.c_void_p, C.c_int, C.POINTER(PsdLabelErrors), i32p, i32p]
+    lib.psd_model_path.restype = C.c_int
+    lib.psd_model_path.argtypes = [C.c_int, C.c_int, C.POINTER(PsdPathProblem), C.c_double, C.c_double, C.POINTER(C.c_void_p)]
+    lib.psd_path_status.restype = C.c_int
+    lib.psd_path_status.argtypes = [C.c_void_p, C.c_int]
+    lib.psd_path_n_models.restype = C.c_int
+    lib.psd_path_n_models.argtypes = [C.c_void_p, C.c_int]
+    lib.psd_path_models.restype = C.c_int
+    lib.psd_path_models.argtypes = [C.c_void_p, C.c_int, C.POINTER(PsdPathModel)]
+    lib.psd_path_target.restype = C.c_int
+    lib.psd_path_target.argtypes = [C.c_void_p, C.c_int, dp, dp, i32p]
+    lib.psd_path_get_stats.restype = C.c_int
+    lib.psd_path_get_stats.argtypes = [C.c_void_p, C.POINTER(PsdPathStats)]
+    lib.psd_path_free.restype = None
+    lib.psd_path_free.argtypes = [C.c_void_p]
     return lib
 
 

@@ -15,6 +15,8 @@
 //                          choose_config()).
 //   fpop_backtrack_kernel  one warp per problem: backtrack_problem() walks the stored records,
 //                          then compacts the segments into one array for a single D2H copy.
+//   label_errors_kernel    (plans with labels only) one warp per problem: label errors of the
+//                          compacted segments (label_errors_gpu.cuh).
 // Problems whose functions outgrow even the per-warp workspace (status 101) are re-run by the same
 // kernel with larger piece lists in global memory; when the store pool is exhausted (status 102)
 // it is grown, then overflows into mapped pinned host memory, and only then are the remaining
@@ -34,6 +36,7 @@
 #include <unordered_map>
 #include <vector>
 #include "dp_params.h"
+#include "label_errors_gpu.cuh"
 #include "rle_gpu.cuh"
 #include "coverage_gpu.cuh"
 #include "plan_internal.h"
@@ -182,6 +185,7 @@ struct psd_plan {
   unsigned char* d_pool = nullptr; unsigned long long pool_bytes = 0, pool_chunk = 0;
   size_t d_rows_cap = 0, d_index_cap = 0, d_prob_cap = 0, d_seg_cap = 0;
   std::vector<std::pair<const RowData*, int64_t>> row_sets;   // distinct row sets of the uploaded problems and their device offsets
+  std::vector<std::pair<const RowData*, int64_t>> packed_row_sets;   // the row sets the pinned staging holds
   unsigned char* d_gws = nullptr; unsigned long long gws_bytes = 0;
   // count-vector problems: raw counts, chromEnd rows, run-length-encoding descriptors
   int *d_raw = nullptr, *d_end = nullptr; size_t d_raw_cap = 0, d_end_cap = 0;
@@ -197,6 +201,14 @@ struct psd_plan {
   unsigned char* d_ring = nullptr; unsigned long long ring_slots = 0, ring_chunk = 0;
   unsigned char* h_ringq = nullptr; unsigned char* d_ringq = nullptr; unsigned int ring_qlen = 0;   // [free_tail 64 B | free_q | done_q]
   cudaStream_t drain_stream = nullptr;
+  // labels of the GPU problems (label_errors_gpu.cuh); n_labels == 0: the plan launches no label kernel
+  int4* d_labels = nullptr; LabelDesc* d_label_desc = nullptr; int *d_label_fp = nullptr, *d_label_fn = nullptr, *d_label_tot = nullptr;
+  int *p_label_fp = nullptr, *p_label_fn = nullptr, *p_label_tot = nullptr;
+  size_t d_label_cap = 0, d_label_prob_cap = 0, p_label_cap = 0, p_label_prob_cap = 0;
+  std::vector<LabelDesc> label_desc;
+  int64_t n_labels = 0;
+  double label_ms = 0;
+  int64_t solve_h2d_bytes = 0, solve_d2h_bytes = 0;   // descriptors, order and status words of the last solve
   // pinned staging
   int32_t *p_weight = nullptr, *p_cov = nullptr;
   DpResult* p_results = nullptr;
@@ -225,6 +237,7 @@ struct psd_plan {
     dfree(d_weight); dfree(d_cov); dfree(d_index); dfree(d_problems); dfree(d_results); dfree(d_order);
     dfree(d_queue); dfree(d_cursors); dfree(d_seg_scratch_off); dfree(d_scratch_row); dfree(d_seg_row);
     dfree(d_scratch_x); dfree(d_seg_x); dfree(d_pool); dfree(d_gws); dfree(d_ring); ring_slots = 0;
+    dfree(d_labels); dfree(d_label_desc); dfree(d_label_fp); dfree(d_label_fn); dfree(d_label_tot); d_label_cap = d_label_prob_cap = 0;
     dfree(d_raw); dfree(d_end); dfree(d_end_off); dfree(d_rle_vecs); dfree(d_tile_vec); dfree(d_tile_state); dfree(d_rle_nrows);
     d_raw_cap = d_end_cap = d_rle_vec_cap = d_tile_cap = 0;
     d_rows_cap = d_index_cap = d_prob_cap = d_seg_cap = 0; pool_bytes = 0; gws_bytes = 0;
@@ -240,6 +253,8 @@ struct psd_plan {
     h_ringq = d_ringq = nullptr; ring_qlen = 0;
     if (drain_stream) { cudaStreamDestroy(drain_stream); drain_stream = nullptr; }
     if (p_raw) cudaFreeHost(p_raw); if (p_rle_nrows) cudaFreeHost(p_rle_nrows);
+    if (p_label_fp) cudaFreeHost(p_label_fp); if (p_label_fn) cudaFreeHost(p_label_fn); if (p_label_tot) cudaFreeHost(p_label_tot);
+    p_label_fp = p_label_fn = p_label_tot = nullptr; p_label_cap = p_label_prob_cap = 0;
     p_raw = nullptr; p_rle_nrows = nullptr; p_raw_cap = p_rle_nrows_cap = 0;
     h_spill = d_spill = nullptr; spill_bytes = 0;
     p_queue_init = nullptr;
@@ -352,6 +367,7 @@ std::vector<HostProblem>& psd_plan_problems(psd_plan* p) { return p->probs; }
 const std::vector<HostProblem>& psd_plan_problems_c(const psd_plan* p) { return p->probs; }
 void psd_plan_invalidate(psd_plan* p) { p->uploaded = false; p->solved = false; p->packed = false; }
 void psd_plan_mark_penalty_changed(psd_plan* p) { p->solved = false; }
+void psd_plan_mark_labels_changed(psd_plan* p) { p->uploaded = false; p->solved = false; }
 const psd_stats& psd_plan_stats_ref(const psd_plan* p) { return p->stats; }
 
 // Predicted store bytes per row (record + index): 16 B header + 8 B index + 40 B per piece pair; 520 B
@@ -390,6 +406,7 @@ int psd_plan_upload_impl(psd_plan* p, void* stream_v) {
         hp.raw_off = total_pos; total_pos += hp.n_pos; n_counts++;
       }
     }
+  if (p->row_sets != p->packed_row_sets) p->packed = false;
   p->rows_plain = 0;
   for (const auto& rs : p->row_sets) p->rows_plain += (int64_t)rs.first->coverage.size();
   for (size_t i = 0; i < p->probs.size(); i++) {
@@ -433,7 +450,7 @@ int psd_plan_upload_impl(psd_plan* p, void* stream_v) {
     };
     if (p->rows_plain > (1 << 22)) parallel_for((int)p->row_sets.size(), pack_one);
     else for (int k = 0; k < (int)p->row_sets.size(); k++) pack_one(k);
-    p->packed = true;
+    p->packed = true; p->packed_row_sets = p->row_sets;
   }
   tr.mark("upload: pack rows");
   // device buffers are grow-only: a plan that is re-uploaded with the same shapes allocates nothing
@@ -552,7 +569,50 @@ int psd_plan_upload_impl(psd_plan* p, void* stream_v) {
     soff[g] = scratch_cursor; scratch_cursor += (unsigned long long)h.n_rows + 1ull;
     eoff[g] = h.from_counts ? (long long)h.row_off : -1;
   }
+  // labels: codes (start, end, kind) packed per GPU problem, in gpu_ids order
+  std::vector<int4> labs;
+  p->label_desc.assign(ng, LabelDesc{0, 0, 0});
+  for (size_t g = 0; g < ng; g++) {
+    const HostProblem& h = p->probs[p->gpu_ids[g]];
+    if (!h.labels) continue;
+    const LabelSet& L = *h.labels;
+    p->label_desc[g].off = (long long)labs.size(); p->label_desc[g].n = (int)L.kind.size();
+    for (size_t k = 0; k < L.kind.size(); k++) labs.push_back(make_int4(L.code_start[k], L.code_end[k], L.kind[k], 0));
+  }
+  p->n_labels = (int64_t)labs.size();
+  if (p->n_labels) {
+    if (labs.size() > p->d_label_cap) {
+      dfree(p->d_labels); dfree(p->d_label_fp); dfree(p->d_label_fn); p->d_label_cap = 0;
+      CK(cudaMalloc(&p->d_labels, sizeof(int4) * labs.size()));
+      CK(cudaMalloc(&p->d_label_fp, sizeof(int) * labs.size()));
+      CK(cudaMalloc(&p->d_label_fn, sizeof(int) * labs.size()));
+      p->d_label_cap = labs.size();
+    }
+    if (ng > p->d_label_prob_cap) {
+      dfree(p->d_label_desc); dfree(p->d_label_tot); p->d_label_prob_cap = 0;
+      CK(cudaMalloc(&p->d_label_desc, sizeof(LabelDesc) * ng));
+      CK(cudaMalloc(&p->d_label_tot, sizeof(int) * 5 * ng));
+      p->d_label_prob_cap = ng;
+    }
+    if (labs.size() > p->p_label_cap) {
+      if (p->p_label_fp) cudaFreeHost(p->p_label_fp); if (p->p_label_fn) cudaFreeHost(p->p_label_fn);
+      p->p_label_fp = p->p_label_fn = nullptr; p->p_label_cap = 0;
+      CK(cudaMallocHost(&p->p_label_fp, sizeof(int) * labs.size()));
+      CK(cudaMallocHost(&p->p_label_fn, sizeof(int) * labs.size()));
+      p->p_label_cap = labs.size();
+    }
+    if (ng > p->p_label_prob_cap) {
+      if (p->p_label_tot) cudaFreeHost(p->p_label_tot);
+      p->p_label_tot = nullptr; p->p_label_prob_cap = 0;
+      CK(cudaMallocHost(&p->p_label_tot, sizeof(int) * 5 * ng));
+      p->p_label_prob_cap = ng;
+    }
+  }
   CK(cudaEventRecord(p->ev[0], st));
+  if (p->n_labels) {
+    CK(cudaMemcpyAsync(p->d_labels, labs.data(), sizeof(int4) * labs.size(), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(p->d_label_desc, p->label_desc.data(), sizeof(LabelDesc) * ng, cudaMemcpyHostToDevice, st));
+  }
   if (plain) {
     CK(cudaMemcpyAsync(p->d_weight, p->p_weight, sizeof(int) * plain, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(p->d_cov, p->p_cov, sizeof(int) * plain, cudaMemcpyHostToDevice, st));
@@ -587,7 +647,8 @@ int psd_plan_upload_impl(psd_plan* p, void* stream_v) {
   float ms = 0; cudaEventElapsedTime(&ms, p->ev[0], p->ev[1]);
   p->stats.h2d_ms = ms;
   p->stats.h2d_bytes = (int64_t)(2 * sizeof(int) * plain + sizeof(int) * total_pos + (sizeof(DpProblem) + 16) * ng +
-                                 sizeof(RleVec) * rvecs.size() + sizeof(int) * tile_vec.size());
+                                 sizeof(RleVec) * rvecs.size() + sizeof(int) * tile_vec.size() +
+                                 (p->n_labels ? sizeof(int4) * labs.size() + sizeof(LabelDesc) * ng : 0));
   if (n_counts) {
     cudaEventElapsedTime(&ms, p->ev[5], p->ev[6]);
     p->stats.rle_ms = ms; p->stats.rle_positions = total_pos;
@@ -820,6 +881,7 @@ int psd_plan_solve_impl(psd_plan* p, void* stream_v) {
   p->results.assign(ng, DpResult());
   p->result_wave.assign(ng, -1);
   p->n_seg_total = 0;
+  p->label_ms = 0; p->solve_h2d_bytes = 0; p->solve_d2h_bytes = 0;
   if (ng == 0) { p->solved = true; return 0; }
   int rc = configure_kernel(p);
   if (rc) return rc;
@@ -836,6 +898,7 @@ int psd_plan_solve_impl(psd_plan* p, void* stream_v) {
     }
     CK(cudaMemcpyAsync(p->d_problems, hp.data(), sizeof(DpProblem) * ng, cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));
+    p->solve_h2d_bytes += (int64_t)(sizeof(DpProblem) * ng);
   }
   const unsigned long long chunk = (unsigned long long)p->opt.chunk_kb << 10;
   std::vector<int> todo(ng);            // problems of the wave about to run (current tier)
@@ -981,6 +1044,7 @@ int psd_plan_solve_impl(psd_plan* p, void* stream_v) {
     CK(cudaMemcpyAsync(p->d_order, todo.data(), sizeof(int) * n, cudaMemcpyHostToDevice, st));
     *p->p_queue_init = grid * wpb;   // slots below this are assigned statically
     CK(cudaMemcpyAsync(p->d_queue, p->p_queue_init, sizeof(int), cudaMemcpyHostToDevice, st));
+    p->solve_h2d_bytes += (int64_t)(sizeof(int) * (n + 1));
     K.queue = p->d_queue;
     CK(cudaMemsetAsync(p->d_cursors, 0, sizeof(unsigned long long), st));   // recycle the store pool
     CK(cudaMemsetAsync(p->d_cursors + 2, 0, sizeof(unsigned long long), st));
@@ -1037,16 +1101,33 @@ int psd_plan_solve_impl(psd_plan* p, void* stream_v) {
     CK(cudaGetLastError());
     CK(cudaEventRecord(p->ev[4], st));
     S.n_launches += 2; S.n_waves++;
+    if (p->n_labels) {
+      LabelParams L;
+      L.results = p->d_results; L.order = p->d_order; L.n_order = n; L.seg_row = p->d_seg_row; L.desc = p->d_label_desc;
+      L.labels = p->d_labels; L.fp = p->d_label_fp; L.fn = p->d_label_fn; L.totals = p->d_label_tot;
+      label_errors_kernel<<<(n + PSD_LABEL_WARPS_PER_BLOCK - 1) / PSD_LABEL_WARPS_PER_BLOCK, PSD_LABEL_WARPS_PER_BLOCK * 32, 0, st>>>(L);
+      CK(cudaGetLastError());
+      CK(cudaEventRecord(p->ev[7], st));
+      S.n_launches++;
+    }
     p->last_hbm_bytes = K.pool.n_chunks * chunk;
     // the wave's status words decide what (if anything) has to be re-run
     CK(cudaMemcpyAsync(p->p_results, p->d_results, sizeof(DpResult) * ng, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(p->p_cursors, p->d_cursors, sizeof(unsigned long long) * 8, cudaMemcpyDeviceToHost, st));
+    p->solve_d2h_bytes += (int64_t)(sizeof(DpResult) * ng + sizeof(unsigned long long) * 8);
+    if (p->n_labels) {   // the label results come back with the status words
+      CK(cudaMemcpyAsync(p->p_label_tot, p->d_label_tot, sizeof(int) * 5 * ng, cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(p->p_label_fp, p->d_label_fp, sizeof(int) * p->n_labels, cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(p->p_label_fn, p->d_label_fn, sizeof(int) * p->n_labels, cudaMemcpyDeviceToHost, st));
+      p->solve_d2h_bytes += (int64_t)(sizeof(int) * (5 * ng + 2 * p->n_labels));
+    }
     tr.mark("solve: launches enqueued");
     CK(cudaStreamSynchronize(st));
     tr.mark("solve: kernels + status D2H");
     float ms = 0;
     cudaEventElapsedTime(&ms, p->ev[2], p->ev[3]); S.dp_ms += ms;
     cudaEventElapsedTime(&ms, p->ev[3], p->ev[4]); S.backtrack_ms += ms;
+    if (p->n_labels) { cudaEventElapsedTime(&ms, p->ev[4], p->ev[7]); p->label_ms += ms; }
     S.store_bytes_written += (int64_t)(std::min<unsigned long long>(p->p_cursors[0], K.pool.n_chunks) * chunk);
     S.store_bytes_spilled_host += (int64_t)(std::min<unsigned long long>(p->p_cursors[2] + (use_ring ? p->p_cursors[5] : 0ull), K.pool.host_chunks) * chunk);
     std::vector<int> exhausted;
@@ -1112,8 +1193,36 @@ int psd_plan_solve_impl(psd_plan* p, void* stream_v) {
   }
   if (sum_rows > 0) p->last_mean_intervals = sum_iv / (2.0 * sum_rows);
   p->n_seg_total = p->p_cursors[1];
+  for (size_t g = 0; g < ng; g++) {   // label errors of the GPU problems
+    HostProblem& h = p->probs[p->gpu_ids[g]];
+    h.label_status = -1; h.label_fp.clear(); h.label_fn.clear();
+    if (!h.labels) continue;
+    h.label_status = p->results[g].status;
+    if (h.label_status != 0) continue;
+    const int* t = p->p_label_tot + 5 * g;
+    h.label_total = psd_label_errors{t[0], t[1], t[2], t[3], t[4]};
+    const LabelDesc& d = p->label_desc[g];
+    h.label_fp.assign(p->p_label_fp + d.off, p->p_label_fp + d.off + d.n);
+    h.label_fn.assign(p->p_label_fn + d.off, p->p_label_fn + d.off + d.n);
+  }
   p->solved = true;
   return 0;
+}
+
+void psd_plan_collect_results(psd_plan* p) {
+  for (size_t g = 0; g < p->gpu_ids.size(); g++) {
+    HostProblem& h = p->probs[p->gpu_ids[g]];
+    const DpResult& r = p->results[g];
+    h.result_status = r.status;
+    if (r.status != 0) continue;
+    h.n_segments = r.n_segments; h.n_equality = r.n_equality;
+    h.best_cost = r.best_cost; h.total_intervals = (double)r.total_intervals; h.max_intervals = r.max_intervals;
+  }
+}
+
+PlanSolveTotals psd_plan_solve_totals(const psd_plan* p) {
+  const psd_stats& S = p->stats;
+  return PlanSolveTotals{S.dp_ms, S.backtrack_ms, p->label_ms, S.rows_solved, S.h2d_bytes + p->solve_h2d_bytes, p->solve_d2h_bytes};
 }
 
 int psd_plan_download_impl(psd_plan* p, void* stream_v) {

@@ -426,6 +426,73 @@ int run_file_batch(int n, const char* const* bedgraphs, const char* const* penal
 
 }  // namespace
 
+// The rows rule of psd_plan_add and psd_model_path.  Returns 0 or the status, *why says which row.
+int check_rows(int64_t n_rows, const int32_t* chromStart, const int32_t* chromEnd, const int32_t* coverage, std::string* why) {
+  char msg[160];
+  if (n_rows <= 0 || n_rows > 0x3fffffff) { snprintf(msg, sizeof msg, "n_rows %lld is outside [1, 0x3fffffff]", (long long)n_rows); *why = msg; return PSD_ERR_ARG; }
+  if (!chromStart || !chromEnd || !coverage) { *why = "a row array is null"; return PSD_ERR_ARG; }
+  // the file path's contract (src/PeakSegFPOPLog.cpp:180-186): rows are contiguous; in addition the
+  // in-memory entry insists on positive widths and non-negative coverage (a zero first width makes
+  // penalty / cumulative weight infinite in the kernel; psd_plan_add_counts rejects negatives too)
+  for (int64_t i = 0; i < n_rows; i++) {
+    if (i > 0 && chromStart[i] != chromEnd[i - 1]) {
+      snprintf(msg, sizeof msg, "row %lld: chromStart %d != chromEnd %d of the row before", (long long)i, chromStart[i], chromEnd[i - 1]);
+      *why = msg; return PSD_ERR_INCONSISTENT_CHROMSTART_CHROMEND;
+    }
+    if (chromEnd[i] <= chromStart[i] || coverage[i] < 0) {
+      snprintf(msg, sizeof msg, "row %lld: empty or negative width, or negative coverage", (long long)i);
+      *why = msg; return PSD_ERR_ARG;
+    }
+  }
+  return 0;
+}
+
+// A row problem (penalty 0) on its own copy of the rows; the rows must have passed check_rows.
+HostProblem make_row_problem(int64_t n_rows, const int32_t* chromStart, const int32_t* chromEnd, const int32_t* coverage) {
+  HostProblem h;
+  h.n_rows = n_rows;
+  h.rows = std::make_shared<RowData>();
+  h.rows->chrom_start.assign(chromStart, chromStart + n_rows);
+  h.rows->chrom_end.assign(chromEnd, chromEnd + n_rows);
+  h.rows->coverage.assign(coverage, coverage + n_rows);
+  finish_rows(*h.rows);
+  finish_problem(h);
+  return h;
+}
+
+// Checks n labels of problem h and converts their ends into codes of h's seg_row units
+// (label_errors_gpu.cuh): 2r for chromEnd[r], 2r - 1 between chromEnd[r - 1] and chromEnd[r]; 2x for
+// count-vector problems.  n == 0 gives no label set.  Returns 0 or PSD_ERR_ARG, *why names the label.
+int make_label_set(const HostProblem& h, int64_t n, const int32_t* start, const int32_t* end, const int32_t* kind,
+                   std::shared_ptr<const LabelSet>* out, std::string* why) {
+  out->reset();
+  char msg[160];
+  if (n < 0 || n > 0x3fffffff) { snprintf(msg, sizeof msg, "n_labels %lld is outside [0, 0x3fffffff]", (long long)n); *why = msg; return PSD_ERR_ARG; }
+  if (n == 0) return 0;
+  if (!start || !end || !kind) { *why = "a label array is null"; return PSD_ERR_ARG; }
+  const int lo = hp_first_start(h), hi = hp_last_end(h);
+  auto L = std::make_shared<LabelSet>();
+  L->start.assign(start, start + n); L->end.assign(end, end + n); L->kind.assign(kind, kind + n);
+  L->code_start.resize(n); L->code_end.resize(n);
+  auto code = [&](int32_t x) -> int32_t {
+    if (h.from_counts) return 2 * x;
+    const std::vector<int32_t>& ce = h.rows->chrom_end;
+    const int32_t r = (int32_t)(std::lower_bound(ce.begin(), ce.end(), x) - ce.begin());
+    return ce[r] == x ? 2 * r : 2 * r - 1;
+  };
+  for (int64_t k = 0; k < n; k++) {
+    if (kind[k] < 0 || kind[k] > 3) { snprintf(msg, sizeof msg, "label %lld: kind %d is not 0..3", (long long)k, kind[k]); *why = msg; return PSD_ERR_ARG; }
+    if (start[k] >= end[k]) { snprintf(msg, sizeof msg, "label %lld: chromStart %d >= chromEnd %d", (long long)k, start[k], end[k]); *why = msg; return PSD_ERR_ARG; }
+    if (start[k] < lo || end[k] > hi) {
+      snprintf(msg, sizeof msg, "label %lld: [%d, %d) is not inside the problem's [%d, %d)", (long long)k, start[k], end[k], lo, hi);
+      *why = msg; return PSD_ERR_ARG;
+    }
+    L->code_start[k] = code(start[k]); L->code_end[k] = code(end[k]);
+  }
+  *out = L;
+  return 0;
+}
+
 extern "C" {
 
 int psd_fpop_disk_batch(int n, const char* const* bedGraph_file_names, const char* const* penalty_strs,
@@ -478,22 +545,13 @@ int psd_plan_add(psd_plan* plan, int64_t n_rows, const int32_t* chromStart, cons
     if (!std::isfinite(penalty)) return -PSD_ERR_PENALTY_NOT_FINITE;
     if (penalty < 0) return -PSD_ERR_PENALTY_NEGATIVE;
   }
-  // the file path's contract (src/PeakSegFPOPLog.cpp:180-186): rows are contiguous; in addition the
-  // in-memory entry insists on positive widths and non-negative coverage (a zero first width makes
-  // penalty / cumulative weight infinite in the kernel; psd_plan_add_counts rejects negatives too)
-  for (int64_t i = 0; i < n_rows; i++) {
-    if (i > 0 && chromStart[i] != chromEnd[i - 1]) return -PSD_ERR_INCONSISTENT_CHROMSTART_CHROMEND;
-    if (chromEnd[i] <= chromStart[i] || coverage[i] < 0) return -PSD_ERR_ARG;
-  }
+  std::string why;
+  const int rc = check_rows(n_rows, chromStart, chromEnd, coverage, &why);
+  if (rc) return -rc;
   std::vector<HostProblem>& v = psd_plan_problems(plan);
-  v.emplace_back();
+  v.push_back(make_row_problem(n_rows, chromStart, chromEnd, coverage));
   HostProblem& h = v.back();
-  h.n_rows = n_rows; h.penalty = penalty; h.penalty_is_inf = penalty_is_inf != 0;
-  h.rows = std::make_shared<RowData>();
-  h.rows->chrom_start.assign(chromStart, chromStart + n_rows);
-  h.rows->chrom_end.assign(chromEnd, chromEnd + n_rows);
-  h.rows->coverage.assign(coverage, coverage + n_rows);
-  finish_rows(*h.rows);
+  h.penalty = penalty; h.penalty_is_inf = penalty_is_inf != 0;
   finish_problem(h);
   psd_plan_invalidate(plan);
   return (int)v.size() - 1;
@@ -528,6 +586,53 @@ int psd_plan_add_counts(psd_plan* plan, int64_t n, const int32_t* counts, double
   h.trivial = h.penalty_is_inf || lo == hi;
   psd_plan_invalidate(plan);
   return (int)v.size() - 1;
+}
+
+int psd_plan_set_labels(psd_plan* plan, int id, int64_t n, const int32_t* chromStart, const int32_t* chromEnd, const int32_t* kind) {
+  if (!plan) { psd_set_last_error("psd_plan_set_labels: plan is null"); return PSD_ERR_ARG; }
+  std::vector<HostProblem>& v = psd_plan_problems(plan);
+  if (id < 0 || id >= (int)v.size()) { psd_set_last_error("psd_plan_set_labels: no problem " + std::to_string(id)); return PSD_ERR_ARG; }
+  std::string why;
+  std::shared_ptr<const LabelSet> L;
+  if (make_label_set(v[id], n, chromStart, chromEnd, kind, &L, &why)) {
+    psd_set_last_error("psd_plan_set_labels: problem " + std::to_string(id) + ": " + why);
+    return PSD_ERR_ARG;
+  }
+  v[id].labels = L;
+  v[id].label_status = -1;
+  psd_plan_mark_labels_changed(plan);
+  return 0;
+}
+
+int psd_plan_label_errors(const psd_plan* plan, int id, psd_label_errors* total, int32_t* fp, int32_t* fn) {
+  if (!plan) return PSD_ERR_ARG;
+  const std::vector<HostProblem>& v = psd_plan_problems_c(plan);
+  if (id < 0 || id >= (int)v.size()) return PSD_ERR_ARG;
+  const HostProblem& h = v[id];
+  if (!h.labels) { psd_set_last_error("psd_plan_label_errors: problem " + std::to_string(id) + " has no labels"); return PSD_ERR_ARG; }
+  if (h.status) return h.status;
+  const LabelSet& L = *h.labels;
+  const size_t n = L.kind.size();
+  if (h.trivial) {   // one segment, no peak: every label that needs a peak misses it
+    psd_label_errors t{};
+    for (size_t k = 0; k < n; k++) {
+      const int miss = L.kind[k] != 0;
+      if (fp) fp[k] = 0;
+      if (fn) fn[k] = miss;
+      t.fn += miss; t.possible_fp += L.kind[k] != 1; t.possible_fn += L.kind[k] != 0;
+    }
+    t.errors = t.fn;
+    if (total) *total = t;
+    return 0;
+  }
+  if (h.label_status != 0) {
+    if (h.label_status < 0) psd_set_last_error("psd_plan_label_errors: problem " + std::to_string(id) + " is not solved");
+    return h.label_status < 0 ? PSD_ERR_ARG : h.label_status;
+  }
+  if (total) *total = h.label_total;
+  if (fp) memcpy(fp, h.label_fp.data(), sizeof(int32_t) * n);
+  if (fn) memcpy(fn, h.label_fn.data(), sizeof(int32_t) * n);
+  return 0;
 }
 
 int psd_plan_size(const psd_plan* plan) { return plan ? (int)psd_plan_problems_c(plan).size() : 0; }

@@ -21,6 +21,13 @@ struct RowData {
   double dmin = 0, dmax = 0;      // log(min coverage), log(max coverage)
 };
 
+// Labels of one problem (psd_plan_set_labels), as given and as codes in the units of the problem's
+// seg_row (label_errors_gpu.cuh).  Shared by the solves of one problem at different penalties.
+struct LabelSet {
+  std::vector<int32_t> start, end, kind;
+  std::vector<int32_t> code_start, code_end;
+};
+
 struct HostProblem {
   int status = 0;                 // reference-style input status (0 ok)
   bool trivial = false;           // one-segment model: penalty Inf or constant coverage
@@ -44,6 +51,11 @@ struct HostProblem {
   double best_cost = 0, total_intervals = 0, max_intervals = 0;
   std::vector<int> seg_row;       // last row of the previous segment, last segment first (-1 for the first)
   std::vector<double> seg_x;      // log-mean per segment
+  // labels and their errors (filled by psd_plan_solve for GPU problems)
+  std::shared_ptr<const LabelSet> labels;
+  int label_status = -1;          // -1 not scored yet, else the solve's status
+  psd_label_errors label_total{};
+  std::vector<int32_t> label_fp, label_fn;
 };
 
 inline int hp_first_start(const HostProblem& h) { return h.from_counts ? 0 : h.rows->chrom_start[0]; }
@@ -97,9 +109,21 @@ const psd_stats& psd_plan_stats_ref(const psd_plan* p);
 int psd_plan_upload_impl(psd_plan* p, void* stream);
 int psd_plan_solve_impl(psd_plan* p, void* stream);
 int psd_plan_download_impl(psd_plan* p, void* stream);
+// what the model-path driver reads back from a solve (model_path.cpp)
+struct PlanSolveTotals { double dp_ms, backtrack_ms, label_ms; int64_t rows_solved, h2d_bytes, d2h_bytes; };
+PlanSolveTotals psd_plan_solve_totals(const psd_plan* p);
+// fills the loss fields of the GPU problems' HostProblem (psd_plan_result) from the solve's status
+// words, without downloading segments
+void psd_plan_collect_results(psd_plan* p);
+void psd_plan_mark_labels_changed(psd_plan* p);
 int psd_plan_store_function_impl(psd_plan* p, int id, int row, int which, int cap, int* n_out, double* hi, int* back_i, double* back_x);
 int psd_device_count_impl();
 int psd_set_option_impl(const char* name, double value);
 int psd_option_devices();                      // option "devices" / env PSD_DEVICES: GPUs one batched file call may use
 void psd_set_last_error(const std::string& s);
+// host_api.cpp: the row and label rules shared by psd_plan_add / psd_plan_set_labels and psd_model_path
+int check_rows(int64_t n_rows, const int32_t* chromStart, const int32_t* chromEnd, const int32_t* coverage, std::string* why);
+HostProblem make_row_problem(int64_t n_rows, const int32_t* chromStart, const int32_t* chromEnd, const int32_t* coverage);
+int make_label_set(const HostProblem& h, int64_t n, const int32_t* start, const int32_t* end, const int32_t* kind,
+                   std::shared_ptr<const LabelSet>* out, std::string* why);
 const std::string& psd_get_last_error();

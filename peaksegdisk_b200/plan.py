@@ -7,6 +7,8 @@ from . import _lib
 LOSS_COLUMNS = ["penalty", "segments", "peaks", "bases", "bedGraph.lines", "mean.pen.cost", "total.loss",
                 "equality.constraints", "mean.intervals", "max.intervals"]   # R/col.name.list.R:12-15
 SEGMENT_COLUMNS = ["chrom", "chromStart", "chromEnd", "status", "mean"]     # R/col.name.list.R:16
+LABEL_KINDS = {"noPeaks": 0, "peaks": 1, "peakStart": 2, "peakEnd": 3}      # PeakError's annotations
+PATH_ERROR_COLUMNS = ["fp", "fn", "possible.fp", "possible.fn", "errors"]
 
 
 def _i32(a):
@@ -83,6 +85,39 @@ class Plan:
         rc = _lib.lib.psd_plan_set_penalty(self._h, pid, 0.0 if is_inf else float(penalty), is_inf)
         if rc:
             raise ValueError(_lib.status_text(rc, penalty=str(penalty)))
+
+    def set_labels(self, pid, labels):
+        """Labels of problem pid: a DataFrame (or dict) with columns chromStart, chromEnd and annotation
+        (noPeaks / peaks / peakStart / peakEnd), 0-based half-open.  They are scored on the device by
+        every later solve (label_errors)."""
+        s, e, k = label_arrays(labels)
+        p32 = C.POINTER(C.c_int32)
+        rc = _lib.lib.psd_plan_set_labels(self._h, pid, len(k), s.ctypes.data_as(p32), e.ctypes.data_as(p32), k.ctypes.data_as(p32))
+        if rc:
+            raise ValueError("peaksegdisk_b200: " + _lib.status_text(rc))
+        if not hasattr(self, "_labels"):
+            self._labels = {}
+        self._labels[pid] = (s, e, k)
+
+    def label_errors(self, pid):
+        """Label errors of problem pid's last solve: (DataFrame with one row per label -- chromStart,
+        chromEnd, annotation, fp, fn, possible.fp, possible.fn -- and a dict of the totals fp, fn,
+        possible.fp, possible.fn, errors)."""
+        import pandas as pd
+        if pid not in getattr(self, "_labels", {}):
+            raise ValueError("peaksegdisk_b200: problem %d has no labels" % pid)
+        s, e, k = self._labels[pid]
+        fp = np.zeros(len(k), np.int32); fn = np.zeros(len(k), np.int32)
+        tot = _lib.PsdLabelErrors()
+        p32 = C.POINTER(C.c_int32)
+        rc = _lib.lib.psd_plan_label_errors(self._h, pid, C.byref(tot), fp.ctypes.data_as(p32), fn.ctypes.data_as(p32))
+        if rc:
+            raise (ValueError if rc == 111 else RuntimeError)("peaksegdisk_b200: " + _lib.status_text(rc))
+        names = np.array(list(LABEL_KINDS))
+        df = pd.DataFrame({"chromStart": s, "chromEnd": e, "annotation": names[k], "fp": fp, "fn": fn,
+                           "possible.fp": (k != 1).astype(np.int32), "possible.fn": (k != 0).astype(np.int32)})
+        return df, {"fp": tot.fp, "fn": tot.fn, "possible.fp": tot.possible_fp, "possible.fn": tot.possible_fn,
+                    "errors": tot.errors}
 
     def _call(self, fn, stream):
         rc = fn(self._h, C.c_void_p(int(stream) if stream else 0))
@@ -211,3 +246,91 @@ def solve_reads_batch(problems, device=-1, stream=0):
     ids = [plan.add(s, e, c, p[4]) for (s, e, c), p in zip(rows, problems)]
     plan.run(stream)
     return plan, ids
+
+
+def label_arrays(labels):
+    """(chromStart, chromEnd, kind) int32 arrays of a label table with columns chromStart, chromEnd and
+    annotation (noPeaks / peaks / peakStart / peakEnd; kind 0..3 in that order)."""
+    try:
+        ann = list(labels["annotation"])
+        s, _ = _coords(labels["chromStart"], "chromStart")
+        e, _ = _coords(labels["chromEnd"], "chromEnd")
+    except KeyError as err:
+        raise ValueError("labels need the columns chromStart, chromEnd and annotation") from err
+    bad = [a for a in ann if a not in LABEL_KINDS]
+    if bad:
+        raise ValueError("label annotation %r is not one of %s" % (bad[0], ", ".join(LABEL_KINDS)))
+    if not len(s) == len(e) == len(ann):
+        raise ValueError("chromStart, chromEnd and annotation must have the same length")
+    return s, e, np.array([LABEL_KINDS[a] for a in ann], np.int32)
+
+
+def model_path_batch(problems, labels=None, pen_min=0.0, pen_max=math.inf, device=-1):
+    """Every model that is optimal for some penalty in [pen_min, pen_max], for each problem
+    (chromStart, chromEnd, coverage), in one psd_model_path call: the pending crossing penalties of all
+    problems are solved together, one batched solve per round (CROPS).  labels: None, or one label
+    DataFrame (or None) per problem; label errors are counted on the device.
+
+    Returns (paths, stats).  paths[i] is {"models": DataFrame, "target": (min.lambda, max.lambda, errors)
+    or None}; the models are sorted by peaks, with penaltyLearning::modelSelection's columns (min.lambda,
+    max.lambda, min.log.lambda, max.log.lambda, penalty, peaks, segments, total.loss) and, for a problem
+    with labels, fp, fn, possible.fp, possible.fn and errors.  A problem whose solve failed has
+    {"status": code, "models": None, "target": None}.  stats is the call's psd_path_stats as a dict."""
+    import pandas as pd
+    problems = list(problems)
+    if labels is None:
+        labels = [None] * len(problems)
+    labels = list(labels)
+    if len(labels) != len(problems):
+        raise ValueError("labels needs one entry (a DataFrame or None) per problem")
+    arr = (_lib.PsdPathProblem * max(1, len(problems)))()
+    keep = []   # the int32 copies must outlive the call
+    p32 = C.POINTER(C.c_int32)
+    for i, ((s, e, c), lab) in enumerate(zip(problems, labels)):
+        s, sp = _i32(s)
+        e, ep = _i32(e)
+        c, cp = _i32(c)
+        if not (len(s) == len(e) == len(c)):
+            raise ValueError("chromStart, chromEnd and coverage must have the same length")
+        keep += [s, e, c]
+        arr[i].n_rows = len(c); arr[i].chromStart = sp; arr[i].chromEnd = ep; arr[i].coverage = cp
+        if lab is not None:
+            ls, le, lk = label_arrays(lab)
+            keep += [ls, le, lk]
+            arr[i].n_labels = len(lk)
+            arr[i].label_start = ls.ctypes.data_as(p32); arr[i].label_end = le.ctypes.data_as(p32)
+            arr[i].label_kind = lk.ctypes.data_as(p32)
+    h = C.c_void_p()
+    rc = _lib.lib.psd_model_path(int(device), len(problems), arr, float(pen_min), float(pen_max), C.byref(h))
+    if rc:
+        raise (ValueError if rc == 111 else RuntimeError)("peaksegdisk_b200: " + _lib.status_text(rc))
+    try:
+        paths = []
+        for i in range(len(problems)):
+            st = _lib.lib.psd_path_status(h, i)
+            if st:
+                paths.append({"status": st, "models": None, "target": None})
+                continue
+            n = _lib.lib.psd_path_n_models(h, i)
+            m = (_lib.PsdPathModel * n)()
+            _lib.lib.psd_path_models(h, i, m)
+            a = np.ctypeslib.as_array(m)
+            lo, hi = a["min_lambda"].copy(), a["max_lambda"].copy()
+            with np.errstate(divide="ignore"):
+                cols = {"min.lambda": lo, "max.lambda": hi, "min.log.lambda": np.log(lo), "max.log.lambda": np.log(hi),
+                        "penalty": a["penalty"].copy(), "peaks": a["peaks"].astype(np.int64),
+                        "segments": a["segments"].astype(np.int64), "total.loss": a["total_loss"].copy()}
+            target = None
+            if labels[i] is not None:
+                for col, f in zip(PATH_ERROR_COLUMNS, ["fp", "fn", "possible_fp", "possible_fn", "errors"]):
+                    cols[col] = a[f].astype(np.int64)
+                tlo, thi, terr = C.c_double(), C.c_double(), C.c_int32()
+                _lib.lib.psd_path_target(h, i, C.byref(tlo), C.byref(thi), C.byref(terr))
+                if terr.value >= 0:
+                    target = (tlo.value, thi.value, terr.value)
+            paths.append({"status": 0, "models": pd.DataFrame(cols), "target": target})
+        st = _lib.PsdPathStats()
+        _lib.lib.psd_path_get_stats(h, C.byref(st))
+        return paths, {name: getattr(st, name) for name, _ in st._fields_}
+    finally:
+        _lib.lib.psd_path_free(h)
