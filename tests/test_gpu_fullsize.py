@@ -25,14 +25,16 @@ def shm(tmp_path_factory):
     shutil.rmtree(d, ignore_errors=True)
 
 
-def _check(psd, cases, paths, mode=0.0):
+def _check(psd, cases, paths, latency_mode=0.0, occupancy_mode=0.0):
     pens = [c["penalty"] for c in cases]
     lib = psd._lib.lib
     try:
-        lib.psd_set_option(b"latency_mode", mode)
+        lib.psd_set_option(b"latency_mode", latency_mode)
+        lib.psd_set_option(b"occupancy_mode", occupancy_mode)
         st = psd.PeakSegFPOP_file_batch(paths, pens)
     finally:
         lib.psd_set_option(b"latency_mode", 0.0)
+        lib.psd_set_option(b"occupancy_mode", 0.0)
     assert st == [0] * len(cases)
     for case, p in zip(cases, paths):
         seg, loss = outputs(p, case["penalty"])
@@ -43,10 +45,12 @@ def _check(psd, cases, paths, mode=0.0):
             os.unlink("%s_penalty=%s%s" % (p, case["penalty"], suf))
 
 
-@pytest.mark.parametrize("mode", [0.0, 2.0], ids=["auto", "throughput-kernel"])
+@pytest.mark.parametrize("mode", [(0.0, 0.0), (2.0, 1.0), (2.0, 2.0)], ids=["auto", "throughput-kernel", "two-block"])
 def test_config2_full_size_vs_reference(psd, shm, mode):
     """Config 2 at its stated size: 8 vectors of 1e5 positions and six of the bench's own vectors
-    (among them the longest and the shortest of the timed batch) x {1e2..1e6} = 70 problems, one call."""
+    (among them the longest and the shortest of the timed batch) x {1e2..1e6} = 70 problems, one call;
+    with the automatic choice, the throughput kernel's one-block build and its two-block build (whose
+    24-piece shared-memory tier these 24-34-piece functions outgrow into the global workspace)."""
     from peaksegdisk_b200 import synth
     cases = golden("golden_fullsize.json")["c2"]
     files = {}
@@ -56,7 +60,7 @@ def test_config2_full_size_vs_reference(psd, shm, mode):
             files[key] = os.path.join(shm, "c2_%d.bedGraph" % key[0])
             if not os.path.exists(files[key]):
                 synth.write_bedgraph(files[key], *synth.poisson_problem(*key))
-    _check(psd, cases, [files[tuple(c["key"])] for c in cases], mode)
+    _check(psd, cases, [files[tuple(c["key"])] for c in cases], *mode)
 
 
 def test_config3_million_row_problem_vs_reference(psd, shm):

@@ -12,10 +12,11 @@ import os
 import numpy as np
 import pytest
 import oracle_bind
-from helpers import ROOT, GOLD, golden, sha, outputs, synth_rows, rows_text, parse_rows, loss_fields, parse_reference_db
+import oracle_checks
+from oracle_checks import check_vs_oracle as _check_vs_oracle, LOSS_RTOL
+from helpers import ROOT, GOLD, golden, sha, outputs, synth_rows, rows_text, parse_rows, loss_fields
 
 pytestmark = pytest.mark.gpu
-LOSS_RTOL = 1e-9   # north_star tolerance for the fp64 total loss
 
 
 @pytest.fixture(scope="module")
@@ -25,16 +26,27 @@ def psd():
     return peaksegdisk_b200
 
 
-@pytest.fixture(autouse=True, params=[0.0, 2.0], ids=["auto", "throughput-kernel"])
+BUILDS = {"auto": (0, 0), "throughput-kernel": (2, 1), "two-block": (2, 2)}   # latency_mode, occupancy_mode
+
+
+@pytest.fixture(autouse=True, params=list(BUILDS))
 def kernel_mode(request, psd):
-    """Every test runs twice: with the automatic choice (small waves go to the latency kernel: one
-    problem per block, one chain per warp) and with the throughput kernel forced (one problem per
-    warp), so both kernels see every parity case."""
-    psd._lib.lib.psd_set_option(b"latency_mode", request.param)
-    os.environ["PSD_LATENCY_MODE"] = str(int(request.param))     # subprocess tools
+    """Every test runs three times: with the automatic choice (small waves go to the latency kernel: one
+    problem per block, one chain per warp), with the throughput kernel's one-block build forced (one
+    problem per warp, one block of 14 warps per SM, 48-piece shared-memory tier) and with its two-block
+    build forced (two blocks per SM, 24-piece tier), so every kernel build sees every parity case.  The
+    environment carries the same choice to the subprocess tools."""
+    lat, occ = BUILDS[request.param]
+    lib = psd._lib.lib
+    lib.psd_set_option(b"latency_mode", float(lat))
+    lib.psd_set_option(b"occupancy_mode", float(occ))
+    os.environ["PSD_LATENCY_MODE"] = str(lat)
+    os.environ["PSD_OCCUPANCY_MODE"] = str(occ)
     yield request.param
-    psd._lib.lib.psd_set_option(b"latency_mode", 0.0)
+    lib.psd_set_option(b"latency_mode", 0.0)
+    lib.psd_set_option(b"occupancy_mode", 0.0)
     os.environ.pop("PSD_LATENCY_MODE", None)
+    os.environ.pop("PSD_OCCUPANCY_MODE", None)
 
 
 def _disk(psd, path, pen, db=None):
@@ -104,23 +116,6 @@ def test_seeded_synthetic_vs_reference_golden_one_batch(psd, tmp_path):
         seg, loss = outputs(p, pen)
         assert loss == case["loss"], (case["kind"], case["key"], pen)
         assert sha(seg) == case["segments_sha256"], (case["kind"], case["key"], pen)
-
-
-def _check_vs_oracle(plan, pid, s, e, c, pen):
-    st, summ, oseg = oracle_bind.solve_rows(s, e, c, pen)
-    assert st == 0
-    r = plan.result(pid)
-    assert r.status == 0
-    got = plan.loss_row(pid)
-    seg = plan.segments(pid)
-    # bit-exact integer outputs
-    assert (got["segments"], got["peaks"], got["equality.constraints"]) == (int(summ[1]), int(summ[2]), int(summ[7]))
-    assert np.array_equal(seg[0], oseg[0]) and np.array_equal(seg[1], oseg[1]) and np.array_equal(seg[2], oseg[2])
-    # fp64 outputs: north_star bar 1e-9; we additionally expect bit equality with the psd_math oracle
-    assert abs(got["total.loss"] - summ[6]) <= LOSS_RTOL * max(1.0, abs(summ[6]))
-    assert got["total.loss"] == summ[6] and got["mean.pen.cost"] == summ[5]
-    assert got["mean.intervals"] == summ[8] and got["max.intervals"] == summ[9]
-    assert np.array_equal(seg[3].view(np.uint64), oseg[3].view(np.uint64))
 
 
 def test_in_memory_batch_vs_oracle_fresh_seeds(psd):
@@ -431,15 +426,8 @@ def test_extreme_values_match_oracle(psd):
     -inf), penalties from 1e-12 to 1e15: the kernels must follow the oracle through every
     inf/underflow corner of the reference's arithmetic."""
     rng = np.random.default_rng(99)
-    probs = []
-    n = 400
-    w = rng.integers(1, 100000000, size=n).astype(np.int64)
-    e = np.cumsum(w) // 64 + np.arange(1, n + 1)          # strictly increasing, below 2^31
-    s = np.concatenate(([0], e[:-1]))
-    big = rng.integers(0, 2000000000, size=n)
-    big[rng.random(n) < 0.3] = 0
-    for pen in (1e-12, 1.0, 1e9, 1e15):
-        probs.append((s.astype(np.int32), e.astype(np.int32), big.astype(np.int32), pen))
+    s, e, big = oracle_checks.extreme_rows(rng)
+    probs = [(s, e, big, pen) for pen in (1e-12, 1.0, 1e9, 1e15)]
     z = np.zeros(300, np.int32); z[100:103] = 7; z[200] = 1
     u = np.arange(300, dtype=np.int32)
     for pen in (0.0, 1e-3, 5.0):
@@ -499,50 +487,34 @@ def test_reference_interface_cpp_runs_the_gpu_solver(psd, tmp_path):
     assert out.returncode == 1 and out.stderr == "Error: unable to write to cost function database file %s\n" % str(tmp_path)
 
 
-def test_store_contents_equal_the_reference_db(psd, tmp_path):
+def test_store_contents_equal_the_reference_db(psd, tmp_path, kernel_mode):
     """Row a10 of the scope table: the HBM cost-function store must hold what the reference's
-    DiskVector holds.  The reference binary (oracle/_ref/ref_fpop, unmodified sources) solves
-    Mono27ac at 10.5 and a synthetic problem and leaves its db; every one of the 2N-1 stored
-    functions -- piece count, max_log_mean, data_i, prev_log_mean of every piece, bit for bit --
-    is read back from the GPU store (psd_plan_store_function) and compared."""
+    DiskVector holds.  The reference binary (oracle/_ref/ref_fpop, unmodified sources) solves the
+    store problems (oracle_checks.store_problems: Mono27ac at 10.5 and 0, synthetic, extreme-value and
+    count-vector problems) and leaves its db; every one of the 2N-1 stored functions -- piece count,
+    max_log_mean, data_i, prev_log_mean of every piece, bit for bit -- is read back from the GPU store
+    (psd_plan_store_function) and compared."""
     import subprocess
     if not os.path.exists(oracle_bind.REF_BIN):
         pytest.skip("oracle/_ref/ref_fpop not built")
-    _store_equals_db(psd, tmp_path, lambda bg, pen: subprocess.call([oracle_bind.REF_BIN, bg, pen, bg + ".db"], stdout=subprocess.DEVNULL))
+    _store_equals_db(psd, tmp_path, kernel_mode,
+                     lambda bg, pen: subprocess.call([oracle_bind.REF_BIN, bg, pen, bg + ".db"], stdout=subprocess.DEVNULL))
 
 
-def test_store_contents_equal_the_oracle_db(psd, tmp_path):
+def test_store_contents_equal_the_oracle_db(psd, tmp_path, kernel_mode):
     """The same comparison against the db the parity oracle writes (oracle/fpop_oracle.cpp, psd_math
     mode: the reference's DiskVector format, which its size matches in tests/golden), so that the store
     is checked function by function on every machine, also where the compiled reference is absent."""
-    _store_equals_db(psd, tmp_path, lambda bg, pen: oracle_bind.oracle_disk(bg, pen, bg + ".db", 1))
+    _store_equals_db(psd, tmp_path, kernel_mode, lambda bg, pen: oracle_bind.oracle_disk(bg, pen, bg + ".db", 1))
 
 
-def _store_equals_db(psd, tmp_path, write_db):
-    """write_db(bedgraph, penalty_str) solves the file and leaves bedgraph + '.db'; returns the status."""
-    from peaksegdisk_b200 import synth
-    _, ms, me, mc = synth.read_bedgraph(os.path.join(GOLD, "Mono27ac_coverage.bedGraph"))
-    probs = [(ms, me, mc, "10.5"), synth.poisson_problem(11, 3000) + ("250",), synth.increasing_problem(150) + ("1000",)]
+def _store_equals_db(psd, tmp_path, build, write_db):
+    probs = oracle_checks.store_problems()
     plan = psd.Plan(0)
-    ids = [plan.add(s, e, c, float(pen)) for (s, e, c, pen) in probs]
+    ids = [p.add(plan) for p in probs]
     plan.run()
-    for k, (pid, (s, e, c, pen)) in enumerate(zip(ids, probs)):
-        bg = str(tmp_path / ("p%d.bedGraph" % k))
-        synth.write_bedgraph(bg, s, e, c)
-        assert write_db(bg, pen) == 0
-        ref = parse_reference_db(bg + ".db", len(c))
-        assert len(ref) == 2 * len(c) - 1 and (0, 0) not in ref      # up_0 does not exist
-        n_pieces = 0
-        for (row, which), (chrom_end, hi, bi, bx) in ref.items():
-            ghi, gbi, gbx = plan.store_function(pid, row, which)
-            assert chrom_end == e[row]
-            assert len(ghi) == len(hi), (k, row, which)
-            assert np.array_equal(ghi.view(np.uint64), hi.view(np.uint64)) and np.array_equal(gbi, bi) and \
-                np.array_equal(gbx.view(np.uint64), bx.view(np.uint64)), (k, row, which)
-            n_pieces += len(hi)
-        assert n_pieces == round(plan.loss_row(pid)["mean.intervals"] * 2 * len(c))
-        hi0, _, _ = plan.store_function(pid, 0, 0)
-        assert len(hi0) == 0
+    for pid, p in zip(ids, probs):
+        oracle_checks.assert_store_equals_db(plan, pid, p, p.db(tmp_path, write_db), build)
 
 
 def test_concurrent_single_problem_calls_from_host_threads(psd, tmp_path):

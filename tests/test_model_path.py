@@ -40,6 +40,18 @@ def option(psd, name, value, default):
         psd._lib.lib.psd_set_option(name.encode(), float(default))
 
 
+@contextlib.contextmanager
+def options(psd, opts):
+    """option() for each (name, value, default) of opts"""
+    with contextlib.ExitStack() as stack:
+        for name, value, default in opts:
+            stack.enter_context(option(psd, name, value, default))
+        yield
+
+
+TWO_BLOCK = [("latency_mode", 2, 0), ("occupancy_mode", 2, 0)]   # the throughput kernel's two-block build, forced
+
+
 def label_df(ls, le, kind):
     return pd.DataFrame({"chromStart": np.asarray(ls, np.int64), "chromEnd": np.asarray(le, np.int64),
                          "annotation": KIND_NAMES[np.asarray(kind)]})
@@ -220,12 +232,14 @@ def test_device_label_errors_equal_the_numpy_oracle(gpu):
         assert tot["possible.fp"] == int((lab[2] != 1).sum()) and tot["possible.fn"] == int((lab[2] != 0).sum())
         want.append((fp, fn))
     assert plan.result(ids[0]).trivial == 1 and plan.result(ids[3]).trivial == 1
-    # the same errors from the latency kernel, from several store waves and from the global piece-list tier
-    for name, value, default in [("latency_mode", 1, 0), ("store_gb", 0.1, 0), ("piece_cap", 8, 48)]:
-        with option(psd, name, value, default), option(psd, "host_spill_gb", 0 if name == "store_gb" else -1, -1):
+    # the same errors from the latency kernel, from the throughput kernel's two-block build, from several
+    # store waves and from the global piece-list tier
+    for name, opts in [("latency", [("latency_mode", 1, 0)]), ("two-block", TWO_BLOCK),
+                       ("store waves", [("store_gb", 0.1, 0), ("host_spill_gb", 0, -1)]), ("piece_cap", [("piece_cap", 8, 48)])]:
+        with options(psd, opts):
             plan2, ids2, _ = solve_with_labels(psd, probs, rng, labels)
         st = plan2.stats()
-        if name == "store_gb":
+        if name == "store waves":
             assert st["n_waves"] > 1, st
         for pid, (fp, fn) in zip(ids2, want):
             df, _ = plan2.label_errors(pid)
@@ -250,6 +264,7 @@ def assert_table_equal(got, want, what):
 
 @pytest.mark.gpu
 def test_model_path_equals_the_oracle_driver_bit_for_bit(gpu):
+    """With the automatic kernel choice and with the throughput kernel's two-block build forced."""
     from peaksegdisk_b200 import synth
     rng = np.random.default_rng(99)
     small, large = [], []
@@ -257,13 +272,13 @@ def test_model_path_equals_the_oracle_driver_bit_for_bit(gpu):
         n = int(rng.integers(200, 2001))
         (small if n <= 500 else large).append(synth.poisson_problem(500 + k, n))
     for probs, lo, hi in [(small, 0.0, math.inf), (large, 10.0, 1e4)]:
-        paths, st = gpu.model_path_batch(probs, pen_min=lo, pen_max=hi)
-        solves = 0
-        for k, (s, e, c) in enumerate(probs):
-            want, rounds, n_solves = path_oracle.crops(path_oracle.oracle_round(s, e, c), lo, hi)
-            assert_table_equal(paths[k]["models"], want, (lo, k))
-            solves += n_solves
-        assert st["solves"] == solves and st["models"] == sum(len(p["models"]) for p in paths)
+        want = [path_oracle.crops(path_oracle.oracle_round(s, e, c), lo, hi) for s, e, c in probs]
+        for build, opts in [("auto", []), ("two-block", TWO_BLOCK)]:
+            with options(gpu, opts):
+                paths, st = gpu.model_path_batch(probs, pen_min=lo, pen_max=hi)
+            for k, (models, rounds, n_solves) in enumerate(want):
+                assert_table_equal(paths[k]["models"], models, (build, lo, k))
+            assert st["solves"] == sum(w[2] for w in want) and st["models"] == sum(len(p["models"]) for p in paths), build
 
 
 @pytest.mark.gpu
