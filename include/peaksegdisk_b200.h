@@ -248,6 +248,37 @@ int psd_coverage_rows(const psd_coverage *cov, int i, int32_t *chromStart, int32
 int psd_coverage_get_stats(const psd_coverage *cov, psd_coverage_stats *out);
 void psd_coverage_free(psd_coverage *cov);
 
+/* ---- per-problem coverage statistics (penalty-learning features) -------------------------------
+ * For one problem the rows give weights w_i = chromEnd_i - chromStart_i and counts c_i; the per-base
+ * vector has B = sum w_i entries (w_i copies of c_i).  The statistics are those of that vector, computed
+ * on the device without expanding it: the quartiles at p = 0, .25, .5, .75, 1 by R's type 7 (h = (B-1) p,
+ * lo = floor(h), g = h - lo; x[lo] when g == 0 or x[lo+1] == x[lo], else (1-g) x[lo] + g x[lo+1] on the
+ * sorted vector x), mean = S1 / B and sd = sqrt((B S2 - S1^2) / (B (B-1))) with S1 = sum w c and
+ * S2 = sum w c^2 in exact integer arithmetic (NaN when B == 1), bases = B and rows = the row count. */
+typedef struct psd_rows {
+  int64_t n_rows;
+  const int32_t *chromStart, *chromEnd, *coverage;   /* rows as for psd_plan_add */
+} psd_rows;
+typedef struct psd_problem_features {
+  double quartile[5];   /* p = 0, .25, .5, .75, 1 (R type 7) */
+  double mean, sd;      /* sd NaN when bases == 1 */
+  int64_t bases, rows;
+} psd_problem_features;
+typedef struct psd_features_stats {
+  double device_ms;     /* CUDA events around H2D + kernels + D2H, summed over waves */
+  double kernel_ms;     /* the histogram and select kernels only */
+  int64_t rows, h2d_bytes, d2h_bytes;
+  int32_t n_problems, n_waves, n_launches;
+} psd_features_stats;
+/* Fills out[0 .. n_problems-1].  Rows are checked on the host before any device work with the rules of
+ * psd_plan_add: a bad problem returns PSD_ERR_ARG (or PSD_ERR_INCONSISTENT_CHROMSTART_CHROMEND for rows
+ * that are not contiguous) and is named in psd_last_error(); so do null arrays and n_problems < 0.  Zero
+ * problems return 0 without touching the device.  Problems go in waves of consecutive problems whose
+ * device buffers fit the "coverage_gb" budget (psd_set_option).  device < 0: the current device.  stats
+ * may be null.  Returns 0, or an error (out's contents are then unspecified). */
+int psd_features(int device, int n_problems, const psd_rows *problems, psd_problem_features *out,
+                 psd_features_stats *stats);
+
 /* Inspection of the cost-function store (replaces DiskVector::read, src/PeakSegFPOPLog.cpp:103-117,
  * for tests and tools): the stored function `which` (0 = up, 1 = down) of bedGraph row `row` of
  * problem id, in the reference's record fields (src/PeakSegFPOPLog.cpp:18-34: max_log_mean, data_i,
@@ -269,8 +300,9 @@ int psd_plan_store_function(psd_plan *plan, int id, int row, int which, int cap,
  * "latency_max_blocks" (16) problems per SM; 1 = always the latency kernel; 2 = never),
  * "devices" (GPUs one psd_fpop_disk_batch call may use: 1 = the current device (default), k = the
  * first k, <= 0 = all; problems are dealt longest-first, one plan and host thread per GPU),
- * "coverage_gb" (device budget of one psd_coverage_from_reads wave: dense per-base buffer, rows and
- * reads; 0 = automatic, half of the free HBM; a problem larger than the budget runs in a wave of its own). */
+ * "coverage_gb" (device budget of one psd_coverage_from_reads or psd_features wave: dense per-base buffer,
+ * rows and reads, or rows and histograms; 0 = automatic, half of the free HBM; a problem larger than the
+ * budget runs in a wave of its own). */
 int psd_set_option(const char *name, double value);
 
 int psd_device_count(void);

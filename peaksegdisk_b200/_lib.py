@@ -71,6 +71,21 @@ class PsdPathStats(C.Structure):
                 ("models", C.c_int32), ("n_problems", C.c_int32)]
 
 
+class PsdRows(C.Structure):
+    _fields_ = [("n_rows", C.c_int64), ("chromStart", C.POINTER(C.c_int32)), ("chromEnd", C.POINTER(C.c_int32)),
+                ("coverage", C.POINTER(C.c_int32))]
+
+
+class PsdProblemFeatures(C.Structure):
+    _fields_ = [("quartile", C.c_double * 5), ("mean", C.c_double), ("sd", C.c_double), ("bases", C.c_int64),
+                ("rows", C.c_int64)]
+
+
+class PsdFeaturesStats(C.Structure):
+    _fields_ = [("device_ms", C.c_double), ("kernel_ms", C.c_double), ("rows", C.c_int64), ("h2d_bytes", C.c_int64),
+                ("d2h_bytes", C.c_int64), ("n_problems", C.c_int32), ("n_waves", C.c_int32), ("n_launches", C.c_int32)]
+
+
 # every symbol include/peaksegdisk_b200.h declares (tests check the library exports all of them)
 C_ABI_SYMBOLS = [
     "psd_fpop_disk", "psd_fpop_disk_batch", "psd_status_message", "psd_last_error", "psd_plan_create",
@@ -79,7 +94,7 @@ C_ABI_SYMBOLS = [
     "psd_set_option", "psd_device_count", "psd_release_cache",
     "psd_coverage_from_reads", "psd_coverage_n_rows", "psd_coverage_rows", "psd_coverage_get_stats", "psd_coverage_free",
     "psd_plan_set_labels", "psd_plan_label_errors", "psd_model_path", "psd_path_status", "psd_path_n_models",
-    "psd_path_models", "psd_path_target", "psd_path_get_stats", "psd_path_free",
+    "psd_path_models", "psd_path_target", "psd_path_get_stats", "psd_path_free", "psd_features",
     "_Z16PeakSegFPOP_diskPcS_S_",   # the reference's own C++-linkage entry (src/PeakSegFPOPLog.h:15)
 ]
 
@@ -160,6 +175,9 @@ def _load():
     lib.psd_path_get_stats.argtypes = [C.c_void_p, C.POINTER(PsdPathStats)]
     lib.psd_path_free.restype = None
     lib.psd_path_free.argtypes = [C.c_void_p]
+    lib.psd_features.restype = C.c_int
+    lib.psd_features.argtypes = [C.c_int, C.c_int, C.POINTER(PsdRows), C.POINTER(PsdProblemFeatures),
+                                 C.POINTER(PsdFeaturesStats)]
     return lib
 
 

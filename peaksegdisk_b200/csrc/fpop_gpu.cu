@@ -6,6 +6,9 @@
 //   reads_scatter_kernel, coverage_scan_kernel, then rle_encode_kernel
 //                          (psd_coverage_from_reads only, not part of a plan) per-base coverage of
 //                          aligned reads and its rows (coverage_gpu.cuh).
+//   features_hist_kernel, features_select_kernel (x 4)
+//                          (psd_features only, not part of a plan) per-problem coverage statistics by
+//                          a weighted radix select over the rows (features_gpu.cuh).
 //   fpop_dp_kernel<W,B>    persistent warps; each warp takes problems (longest first) from an atomic
 //                          queue and runs dp_run_queue() (fpop_warp.cuh): the whole DP of one
 //                          (bedGraph x penalty), piece lists in shared memory (moving to a per-warp
@@ -39,6 +42,7 @@
 #include "label_errors_gpu.cuh"
 #include "rle_gpu.cuh"
 #include "coverage_gpu.cuh"
+#include "features_gpu.cuh"
 #include "plan_internal.h"
 
 #define PSD_MAX_WARPS_PER_BLOCK 16   /* __launch_bounds__(512): 128 registers per thread (fewer registers only add spills; 14-16 warps fit shared memory) */
@@ -1563,6 +1567,213 @@ int psd_coverage_from_reads_impl(int device, int n, const psd_reads* P, psd_cove
   emit_empty_until(n);
   S.rows = (int64_t)C->count.size();
   *out = C.release();
+  return 0;
+}
+
+// ---- per-problem coverage statistics (psd_features, features_gpu.cuh) ---------------------------------
+namespace {
+struct FeatScratch {
+  unsigned char* d_arena = nullptr;
+  int32_t *p_w = nullptr, *p_c = nullptr;   // weight and count rows of a wave
+  cudaEvent_t ev[4]; bool ev_ok = false;
+  ~FeatScratch() {
+    if (d_arena) cudaFree(d_arena);
+    if (p_w) cudaFreeHost(p_w); if (p_c) cudaFreeHost(p_c);
+    if (ev_ok) for (auto& e : ev) cudaEventDestroy(e);
+  }
+};
+
+struct FeatJob {
+  int64_t bases;
+  int64_t rank[PSD_FEAT_SEL];   // the distinct ranks of x the interior quartiles need, ascending
+  int n_sel;
+  int64_t n_tiles;
+};
+
+// device bytes of a wave (the arena is carved in this order, see psd_features_impl)
+size_t feat_wave_bytes(int64_t n_probs, int64_t rows, int64_t tiles, int64_t sels) {
+  return 2 * cov_align(4 * rows) + cov_align(sizeof(FeatProblem) * n_probs) + cov_align(4 * tiles) +
+         cov_align(sizeof(FeatSel) * sels) + cov_align(2048 * sels) + cov_align(sizeof(FeatSums) * n_probs) + cov_align(4);
+}
+
+// R's type-7 quantile at p from x[lo] and x[lo + 1] (h = (B - 1) p, lo = floor(h), g = h - lo); every
+// step is exact in fp64 for int32 counts and B < 2^32
+void feat_type7(int64_t B, double p, double* h, int64_t* lo, double* g) {
+  *h = (double)(B - 1) * p;
+  *lo = (int64_t)std::floor(*h);
+  *g = *h - (double)*lo;
+}
+}  // namespace
+
+// Host checks (check_rows, before any device work), then waves of consecutive problems that fit the
+// "coverage_gb" budget: H2D of weight and count, four histogram + select passes, D2H of the sums and
+// the selected counts; the host turns the integers into the features.
+int psd_features_impl(int device, int n, const psd_rows* P, psd_problem_features* out, psd_features_stats* stats) {
+  psd_features_stats S;
+  memset(&S, 0, sizeof S);
+  if (stats) *stats = S;
+  if (n < 0 || (n > 0 && (!P || !out))) { g_last_error = "psd_features: n_problems < 0, or problems or out is null"; return PSD_ERR_ARG; }
+  std::vector<std::string> err(n);
+  std::vector<int> code(n, 0);
+  auto check = [&](int k) { code[k] = check_rows(P[k].n_rows, P[k].chromStart, P[k].chromEnd, P[k].coverage, &err[k]); };
+  int64_t all_rows = 0;
+  for (int k = 0; k < n; k++) all_rows += P[k].n_rows > 0 ? P[k].n_rows : 0;
+  if (all_rows > (1 << 22)) parallel_for(n, check);
+  else for (int k = 0; k < n; k++) check(k);
+  for (int k = 0; k < n; k++)
+    if (code[k]) { g_last_error = "psd_features: problem " + std::to_string(k) + ": " + err[k]; return code[k]; }
+  if (n == 0) return 0;
+  S.n_problems = n;
+
+  std::vector<FeatJob> jobs(n);
+  for (int k = 0; k < n; k++) {
+    FeatJob& J = jobs[k];
+    J.bases = (int64_t)P[k].chromEnd[P[k].n_rows - 1] - P[k].chromStart[0];
+    J.n_tiles = (P[k].n_rows + PSD_RLE_TILE - 1) / PSD_RLE_TILE;
+    J.n_sel = 0;
+    for (double p : {0.25, 0.5, 0.75}) {
+      double h, g; int64_t lo;
+      feat_type7(J.bases, p, &h, &lo, &g);
+      for (int64_t r : {lo, g != 0 ? lo + 1 : lo})
+        if (std::find(J.rank, J.rank + J.n_sel, r) == J.rank + J.n_sel) J.rank[J.n_sel++] = r;
+    }
+    std::sort(J.rank, J.rank + J.n_sel);
+  }
+  int ndev = 0;
+  if (!cuda_ok(cudaGetDeviceCount(&ndev), "cudaGetDeviceCount")) return PSD_ERR_CUDA;
+  if (ndev == 0) { g_last_error = "no CUDA device"; return PSD_ERR_CUDA; }
+  if (device < 0) CK(cudaGetDevice(&device));
+  CK(cudaSetDevice(device));
+  cudaDeviceProp prop;
+  CK(cudaGetDeviceProperties(&prop, device));
+  if (prop.major < 10) { g_last_error = "peaksegdisk_b200 is built for sm_100a only"; return PSD_ERR_CUDA; }
+  FeatScratch X;
+  for (auto& e : X.ev) CK(cudaEventCreate(&e));
+  X.ev_ok = true;
+  // waves: consecutive problems while their footprint fits the budget (a problem larger than it runs alone)
+  size_t free_b = 0, total_b = 0;
+  CK(cudaMemGetInfo(&free_b, &total_b));
+  const double gb = current_options().coverage_gb;
+  const size_t budget = gb > 0 ? (size_t)(gb * (double)(1ull << 30)) : free_b / 2;
+  std::vector<std::pair<int, int>> waves;   // [first problem, end problem)
+  size_t arena = 0, max_rows = 0;
+  for (int k0 = 0; k0 < n;) {
+    int k1 = k0;
+    int64_t rows = 0, tiles = 0, sels = 0;
+    size_t bytes = 0;
+    for (; k1 < n; k1++) {
+      const size_t b = feat_wave_bytes(k1 - k0 + 1, rows + P[k1].n_rows, tiles + jobs[k1].n_tiles, sels + jobs[k1].n_sel);
+      if (k1 > k0 && b > budget) break;
+      rows += P[k1].n_rows; tiles += jobs[k1].n_tiles; sels += jobs[k1].n_sel; bytes = b;
+    }
+    waves.push_back({k0, k1});
+    arena = std::max(arena, bytes); max_rows = std::max(max_rows, (size_t)rows);
+    k0 = k1;
+  }
+  CK(cudaMalloc(&X.d_arena, arena));
+  CK(cudaMallocHost(&X.p_w, 4 * max_rows));
+  CK(cudaMallocHost(&X.p_c, 4 * max_rows));
+  const cudaStream_t st = 0;
+  for (const auto& w : waves) {
+    const int np = w.second - w.first;
+    std::vector<FeatProblem> probs(np);
+    std::vector<FeatSel> sel;
+    std::vector<int> tile_prob;
+    int64_t rows = 0;
+    for (int j = 0; j < np; j++) {
+      const FeatJob& J = jobs[w.first + j];
+      FeatProblem& q = probs[j];
+      q.row_off = rows; q.n_rows = (int)P[w.first + j].n_rows; q.tile0 = (int)tile_prob.size();
+      q.sel0 = (int)sel.size(); q.n_sel = J.n_sel;
+      tile_prob.insert(tile_prob.end(), (size_t)J.n_tiles, j);
+      for (int s = 0; s < J.n_sel; s++) sel.push_back(FeatSel{(unsigned long long)J.rank[s], 0u, q.sel0});
+      rows += q.n_rows;
+    }
+    const int n_tiles = (int)tile_prob.size(), n_sel = (int)sel.size();
+    auto stage = [&](int j) {
+      const psd_rows& q = P[w.first + j];
+      int32_t* pw = X.p_w + probs[j].row_off;
+      for (int64_t i = 0; i < q.n_rows; i++) pw[i] = q.chromEnd[i] - q.chromStart[i];
+      memcpy(X.p_c + probs[j].row_off, q.coverage, 4 * (size_t)q.n_rows);
+    };
+    if (rows > (1 << 22)) parallel_for(np, stage);
+    else for (int j = 0; j < np; j++) stage(j);
+    std::vector<FeatSums> sums(np, FeatSums{0ull, 0ull, 0ull, 0xffffffffu, 0u});
+    // carve the arena (the order feat_wave_bytes() counts)
+    unsigned char* a = X.d_arena;
+    auto carve = [&](size_t b) { unsigned char* r = a; a += cov_align(b); return r; };
+    int* d_w = (int*)carve(4 * rows);
+    int* d_c = (int*)carve(4 * rows);
+    FeatProblem* d_probs = (FeatProblem*)carve(sizeof(FeatProblem) * np);
+    int* d_tile_prob = (int*)carve(4 * (size_t)n_tiles);
+    FeatSel* d_sel = (FeatSel*)carve(sizeof(FeatSel) * n_sel);
+    unsigned long long* d_hist = (unsigned long long*)carve(2048 * (size_t)n_sel);
+    FeatSums* d_sums = (FeatSums*)carve(sizeof(FeatSums) * np);
+    int* d_err = (int*)carve(4);
+    CK(cudaEventRecord(X.ev[0], st));
+    CK(cudaMemcpyAsync(d_w, X.p_w, 4 * rows, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_c, X.p_c, 4 * rows, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_probs, probs.data(), sizeof(FeatProblem) * np, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_tile_prob, tile_prob.data(), 4 * (size_t)n_tiles, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_sel, sel.data(), sizeof(FeatSel) * n_sel, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_sums, sums.data(), sizeof(FeatSums) * np, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(X.ev[1], st));
+    CK(cudaMemsetAsync(d_hist, 0, 2048 * (size_t)n_sel, st));
+    CK(cudaMemsetAsync(d_err, 0, 4, st));
+    for (int pass = 0; pass < 4; pass++) {
+      FeatHistParams H;
+      H.probs = d_probs; H.tile_prob = d_tile_prob; H.n_tiles = n_tiles; H.weight = d_w; H.count = d_c;
+      H.sel = d_sel; H.hist = d_hist; H.sums = d_sums;
+      H.shift = 24 - 8 * pass; H.mask = pass == 0 ? 0u : 0xffffffffu << (H.shift + 8);
+      if (pass == 0) features_hist_kernel<true><<<n_tiles, PSD_RLE_WARPS * 32, 0, st>>>(H);
+      else features_hist_kernel<false><<<n_tiles, PSD_RLE_WARPS * 32, 0, st>>>(H);
+      CK(cudaGetLastError());
+      FeatSelectParams Z;
+      Z.probs = d_probs; Z.n_probs = np; Z.sel = d_sel; Z.hist = d_hist; Z.shift = H.shift; Z.error = d_err;
+      features_select_kernel<<<(np + 7) / 8, 256, 0, st>>>(Z);
+      CK(cudaGetLastError());
+      S.n_launches += 2;
+    }
+    CK(cudaEventRecord(X.ev[2], st));
+    int h_err = 0;
+    CK(cudaMemcpyAsync(sums.data(), d_sums, sizeof(FeatSums) * np, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(sel.data(), d_sel, sizeof(FeatSel) * n_sel, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&h_err, d_err, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaEventRecord(X.ev[3], st));
+    CK(cudaStreamSynchronize(st));
+    if (h_err) { g_last_error = "device features: a rank fell outside its histogram"; return PSD_ERR_INTERNAL; }
+    float t03 = 0, t12 = 0;
+    cudaEventElapsedTime(&t03, X.ev[0], X.ev[3]); cudaEventElapsedTime(&t12, X.ev[1], X.ev[2]);
+    S.device_ms += t03; S.kernel_ms += t12;
+    S.rows += rows; S.n_waves++;
+    S.h2d_bytes += 8 * rows + (int64_t)(sizeof(FeatProblem) + sizeof(FeatSums)) * np + 4 * (int64_t)n_tiles + (int64_t)sizeof(FeatSel) * n_sel;
+    S.d2h_bytes += (int64_t)sizeof(FeatSums) * np + (int64_t)sizeof(FeatSel) * n_sel + 4;
+    for (int j = 0; j < np; j++) {
+      const FeatJob& J = jobs[w.first + j];
+      const FeatSums& U = sums[j];
+      auto x_at = [&](int64_t r) { return (double)sel[probs[j].sel0 + (std::find(J.rank, J.rank + J.n_sel, r) - J.rank)].prefix; };
+      psd_problem_features& F = out[w.first + j];
+      const int64_t B = J.bases;
+      F.quartile[0] = (double)U.min;
+      F.quartile[4] = (double)U.max;
+      const double ps[3] = {0.25, 0.5, 0.75};
+      for (int t = 0; t < 3; t++) {
+        double h, g; int64_t lo;
+        feat_type7(B, ps[t], &h, &lo, &g);
+        const double x0 = x_at(lo);
+        if (g == 0) { F.quartile[t + 1] = x0; continue; }
+        const double x1 = x_at(lo + 1);
+        F.quartile[t + 1] = x1 == x0 ? x0 : (1 - g) * x0 + g * x1;
+      }
+      F.mean = (double)(int64_t)U.s1 / (double)B;
+      const unsigned __int128 s2 = ((unsigned __int128)U.s2_hi << 64) | U.s2_lo;
+      const unsigned __int128 V = (unsigned __int128)(uint64_t)B * s2 - (unsigned __int128)U.s1 * U.s1;
+      F.sd = B == 1 ? NAN : std::sqrt((double)V / ((double)B * (double)(B - 1)));
+      F.bases = B;
+      F.rows = P[w.first + j].n_rows;
+    }
+  }
+  if (stats) *stats = S;
   return 0;
 }
 

@@ -784,6 +784,10 @@ int psd_coverage_get_stats(const psd_coverage* cov, psd_coverage_stats* out) {
 
 void psd_coverage_free(psd_coverage* cov) { delete cov; }
 
+int psd_features(int device, int n_problems, const psd_rows* problems, psd_problem_features* out, psd_features_stats* stats) {
+  return psd_features_impl(device, n_problems, problems, out, stats);
+}
+
 int psd_set_option(const char* name, double value) { return name ? psd_set_option_impl(name, value) : PSD_ERR_ARG; }
 int psd_device_count(void) { return psd_device_count_impl(); }
 void psd_release_cache(void) { psd_plan_drop_parked(); }

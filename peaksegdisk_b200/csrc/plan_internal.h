@@ -94,6 +94,7 @@ struct psd_coverage {
   psd_coverage_stats stats;
 };
 int psd_coverage_from_reads_impl(int device, int n_problems, const psd_reads* problems, psd_coverage** out);
+int psd_features_impl(int device, int n_problems, const psd_rows* problems, psd_problem_features* out, psd_features_stats* stats);
 
 struct psd_plan;
 psd_plan* psd_plan_create_impl(int device);

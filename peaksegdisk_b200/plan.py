@@ -248,6 +248,49 @@ def solve_reads_batch(problems, device=-1, stream=0):
     return plan, ids
 
 
+FEATURE_NAMES = ["quartile.0%", "quartile.25%", "quartile.50%", "quartile.75%", "quartile.100%", "mean", "sd",
+                 "bases", "data"]   # PeakSegPipeline's problem.features
+FEATURE_COLUMNS = FEATURE_NAMES + [pre + f for pre in ("log+1.", "log.", "log.log.") for f in FEATURE_NAMES]
+
+
+def problem_features(problems, device=-1, return_stats=False):
+    """problems: iterable of (chromStart, chromEnd, coverage) rows.  The coverage statistics of each
+    problem's per-base vector (each row repeated chromEnd - chromStart times), computed on the device in
+    ONE psd_features call without expanding the rows (features_gpu.cuh).  Returns a DataFrame with one
+    row per problem and 36 columns: quartile.0% .. quartile.100% (R's type 7), mean, sd (NaN for one
+    base), bases and data (rows), then the same nine with the prefixes log+1., log. and log.log. (-inf for
+    the log of 0, NaN for the log of a negative).  With return_stats, also the call's psd_features_stats
+    as a dict."""
+    import pandas as pd
+    problems = list(problems)
+    arr = (_lib.PsdRows * max(1, len(problems)))()
+    keep = []   # the int32 copies must outlive the call
+    for i, (s, e, c) in enumerate(problems):
+        s, sp = _i32(s)
+        e, ep = _i32(e)
+        c, cp = _i32(c)
+        if not (len(s) == len(e) == len(c)):
+            raise ValueError("chromStart, chromEnd and coverage must have the same length")
+        keep += [s, e, c]
+        arr[i].n_rows = len(c); arr[i].chromStart = sp; arr[i].chromEnd = ep; arr[i].coverage = cp
+    out = (_lib.PsdProblemFeatures * max(1, len(problems)))()
+    st = _lib.PsdFeaturesStats()
+    rc = _lib.lib.psd_features(int(device), len(problems), arr, out, C.byref(st))
+    if rc in (111, 6):   # PSD_ERR_ARG, PSD_ERR_INCONSISTENT_CHROMSTART_CHROMEND: the message names the problem
+        raise ValueError("peaksegdisk_b200: " + _lib.lib.psd_last_error().decode())
+    if rc:
+        raise RuntimeError("peaksegdisk_b200: " + _lib.status_text(rc))
+    a = np.ctypeslib.as_array(out)[:len(problems)]
+    base = np.column_stack([a["quartile"].reshape(-1, 5), a["mean"], a["sd"], a["bases"].astype(np.float64),
+                            a["rows"].astype(np.float64)]) if len(problems) else np.zeros((0, 9))
+    with np.errstate(divide="ignore", invalid="ignore"):
+        x = np.hstack([base, np.log(base + 1), np.log(base), np.log(np.log(base))])
+    df = pd.DataFrame(x, columns=FEATURE_COLUMNS)
+    if return_stats:
+        return df, {name: getattr(st, name) for name, _ in st._fields_}
+    return df
+
+
 def label_arrays(labels):
     """(chromStart, chromEnd, kind) int32 arrays of a label table with columns chromStart, chromEnd and
     annotation (noPeaks / peaks / peakStart / peakEnd; kind 0..3 in that order)."""
