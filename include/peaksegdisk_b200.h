@@ -279,6 +279,84 @@ typedef struct psd_features_stats {
 int psd_features(int device, int n_problems, const psd_rows *problems, psd_problem_features *out,
                  psd_features_stats *stats);
 
+/* ---- joint single-peak models of many samples (the model of PeakSegJoint, solved exactly) -------------
+ * A problem is one region [region_start, region_end) with S samples (1 <= S <= 256) whose rows (the rules of
+ * psd_plan_add) tile the region exactly, and a bin width bin_bases >= 1.
+ *   Grid: g_k = region_start + k bin_bases for k = 0..N-1 and g_N = region_end, N = ceil(length / bin_bases)
+ *   (the last bin may be shorter).  N is at most PSD_JOINT_MAX_BINS: a problem's work grows as N^2 S (about
+ *   1.4e11 pair x sample evaluations at the cap with 256 samples), and pair indices stay in 32 bits.
+ *   Sums: C_s(i, j) = the sum of sample s's counts over the bases of [g_i, g_j) (exact int64), W(i, j) = g_j - g_i.
+ *   Segment loss: L_s(i, j) = C - C log(C / W) in double (0 when C = 0); the flat model of s has L1_s = L_s(0, N),
+ *   and flat = the sum of L1_s in sample order.
+ *   Peak (a, b), 1 <= a < b <= N-1: sample s can carry it only if C_s(a,b) W(0,a) > C_s(0,a) W(a,b) and
+ *   C_s(a,b) W(b,N) > C_s(b,N) W(a,b) (exact integers: its peak mean is strictly above both flank means);
+ *   then L3_s = (L_s(0,a) + L_s(a,b)) + L_s(b,N) and r_s = L1_s - L3_s.
+ *   Model k at (a, b): the first k feasible samples in the order (r desc, sample index asc) carry the peak;
+ *   loss_k(a, b) = flat - R_k, R_k their reductions added one after the other in that order (+inf when
+ *   fewer than k samples are feasible).
+ *   Model k (k = 0..S): the minimum of loss_k over all peaks, ties to the smaller a, then the smaller b.  Model 0
+ *   is the flat model without a peak; a k that no peak reaches has no model.
+ *   Selection: argmin_k loss_k + lambda k, lambda in [0, inf).  The selectable models are the corners of the
+ *   lower convex hull of (k, loss_k), added by increasing k, a corner being dropped unless the breakpoint
+ *   (loss_i - loss_j) / (j - i) with the corner before it is strictly larger than with the next one and
+ *   strictly positive.  A selectable model gets [min_lambda, max_lambda] from its breakpoints (model 0:
+ *   max_lambda = inf; the selectable model with the most peaks: min_lambda = 0); the others get NaN.
+ *   Labels (optional, per sample, the kinds and rules of psd_plan_set_labels): in model k each peaked sample has
+ *   the one peak [g_a, g_b) and the others none; fp / fn / possible_fp / possible_fn / errors are summed over
+ *   all samples' labels, and the target interval is psd_model_path's, over the selectable models.
+ * The device computes the minima (joint_gpu.cuh); the host recomputes each winner's samples and loss in the same
+ * arithmetic and requires the same bits (PSD_ERR_INTERNAL otherwise).  This is not PeakSegJoint's binned search:
+ * it is the exact optimum over every peak of the grid. */
+#define PSD_JOINT_MAX_SAMPLES 256
+#define PSD_JOINT_MAX_BINS 32768
+typedef struct psd_joint_sample {
+  int64_t n_rows;                                    /* rows as for psd_plan_add */
+  const int32_t *chromStart, *chromEnd, *coverage;
+  int64_t n_labels;                                  /* labels as for psd_plan_set_labels (0: none) */
+  const int32_t *label_start, *label_end, *label_kind;
+} psd_joint_sample;
+typedef struct psd_joint_problem {
+  int32_t region_start, region_end;                  /* every sample's rows tile exactly this region */
+  int32_t bin_bases;                                 /* bin width, >= 1 */
+  int32_t n_samples;                                 /* S, 1..PSD_JOINT_MAX_SAMPLES */
+  const psd_joint_sample *samples;
+} psd_joint_problem;
+typedef struct psd_joint_model {
+  double total_loss;
+  double min_lambda, max_lambda;   /* NaN when not selectable */
+  int32_t peaks;                   /* k, the number of samples with the peak */
+  int32_t peak_start, peak_end;    /* [g_a, g_b); -1 for k = 0 */
+  int32_t selectable;
+  int32_t fp, fn, possible_fp, possible_fn, errors;   /* sums over all samples' labels; zero without labels */
+  int32_t pad_;
+} psd_joint_model;
+typedef struct psd_joint psd_joint;
+typedef struct psd_joint_stats {
+  double device_ms;                /* CUDA events around H2D + kernels + D2H, summed over waves */
+  double kernel_ms;                /* the flank, flat, pair and reduce kernels only */
+  int64_t samples;                 /* sum of S over the problems */
+  int64_t pair_sample_evals;       /* sum of S (N-1)(N-2)/2: the (peak, sample) pairs scored on the device */
+  int64_t h2d_bytes, d2h_bytes;
+  int32_t n_problems, n_waves, n_launches, pad_;
+} psd_joint_stats;
+/* Solves n_problems problems.  Inputs are checked on the host before any device work: S outside 1..256, a null
+ * sample array, rows that break psd_plan_add's rules or do not tile the problem's region, bin_bases < 1, N over
+ * PSD_JOINT_MAX_BINS and bad labels return PSD_ERR_ARG, and psd_last_error() names the problem and the sample.
+ * Zero problems never touch the device.  Problems go in waves whose device buffers fit the "coverage_gb" budget
+ * (psd_set_option); a problem larger than the budget runs alone.  device < 0: the current device.  Returns 0
+ * and *out (free it with psd_joint_free), or an error and no handle. */
+int psd_joint_models(int device, int n_problems, const psd_joint_problem *problems, psd_joint **out);
+int psd_joint_n_models(const psd_joint *h, int i);   /* models of problem i (k that have one); -1 if i is out of range */
+/* Copies problem i's models, k ascending; the array needs psd_joint_n_models entries. */
+int psd_joint_model_table(const psd_joint *h, int i, psd_joint_model *models);
+/* in_peak[s] = 1 if sample s carries the peak in problem i's model with k peaked samples (S entries); PSD_ERR_ARG
+ * if that model does not exist. */
+int psd_joint_samples(const psd_joint *h, int i, int k, uint8_t *in_peak);
+/* Problem i's target interval: *errors = -1 (and NaN penalties) when no sample of it has labels. */
+int psd_joint_target(const psd_joint *h, int i, double *min_lambda, double *max_lambda, int32_t *errors);
+int psd_joint_get_stats(const psd_joint *h, psd_joint_stats *out);
+void psd_joint_free(psd_joint *h);
+
 /* Inspection of the cost-function store (replaces DiskVector::read, src/PeakSegFPOPLog.cpp:103-117,
  * for tests and tools): the stored function `which` (0 = up, 1 = down) of bedGraph row `row` of
  * problem id, in the reference's record fields (src/PeakSegFPOPLog.cpp:18-34: max_log_mean, data_i,
@@ -300,9 +378,9 @@ int psd_plan_store_function(psd_plan *plan, int id, int row, int which, int cap,
  * "latency_max_blocks" (16) problems per SM; 1 = always the latency kernel; 2 = never),
  * "devices" (GPUs one psd_fpop_disk_batch call may use: 1 = the current device (default), k = the
  * first k, <= 0 = all; problems are dealt longest-first, one plan and host thread per GPU),
- * "coverage_gb" (device budget of one psd_coverage_from_reads or psd_features wave: dense per-base buffer,
- * rows and reads, or rows and histograms; 0 = automatic, half of the free HBM; a problem larger than the
- * budget runs in a wave of its own). */
+ * "coverage_gb" (device budget of one psd_coverage_from_reads, psd_features or psd_joint_models wave: dense
+ * per-base buffer, rows and reads; rows and histograms; or prefix sums, flank losses and per-chunk candidates;
+ * 0 = automatic, half of the free HBM; a problem larger than the budget runs in a wave of its own). */
 int psd_set_option(const char *name, double value);
 
 int psd_device_count(void);

@@ -7,10 +7,11 @@ from . import _lib
 from .api import (PeakSegFPOP_file, PeakSegFPOP_file_batch, PeakSegFPOP_dir, PeakSegFPOP_df, PeakSegFPOP_vec,
                   PeakSegFPOP_vec_batch, coverage_from_reads,
                   sequentialSearch_dir, sequentialSearch_batch, writeBedGraph, col_name_list, r_paste)
-from .plan import Plan, solve_batch, solve_counts_batch, solve_reads_batch, model_path_batch, problem_features
+from .plan import (Plan, solve_batch, solve_counts_batch, solve_reads_batch, model_path_batch, problem_features,
+                   joint_models_batch)
 from .learn import IntervalRegressionCV
 
 __all__ = ["PeakSegFPOP_file", "PeakSegFPOP_file_batch", "PeakSegFPOP_dir", "PeakSegFPOP_df", "PeakSegFPOP_vec", "PeakSegFPOP_vec_batch",
            "sequentialSearch_dir", "sequentialSearch_batch", "writeBedGraph", "col_name_list", "r_paste", "Plan", "solve_batch",
            "solve_counts_batch", "coverage_from_reads", "solve_reads_batch", "model_path_batch",
-           "problem_features", "IntervalRegressionCV"]
+           "problem_features", "joint_models_batch", "IntervalRegressionCV"]

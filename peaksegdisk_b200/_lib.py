@@ -86,6 +86,30 @@ class PsdFeaturesStats(C.Structure):
                 ("d2h_bytes", C.c_int64), ("n_problems", C.c_int32), ("n_waves", C.c_int32), ("n_launches", C.c_int32)]
 
 
+class PsdJointSample(C.Structure):
+    _fields_ = [("n_rows", C.c_int64), ("chromStart", C.POINTER(C.c_int32)), ("chromEnd", C.POINTER(C.c_int32)),
+                ("coverage", C.POINTER(C.c_int32)), ("n_labels", C.c_int64), ("label_start", C.POINTER(C.c_int32)),
+                ("label_end", C.POINTER(C.c_int32)), ("label_kind", C.POINTER(C.c_int32))]
+
+
+class PsdJointProblem(C.Structure):
+    _fields_ = [("region_start", C.c_int32), ("region_end", C.c_int32), ("bin_bases", C.c_int32), ("n_samples", C.c_int32),
+                ("samples", C.POINTER(PsdJointSample))]
+
+
+class PsdJointModel(C.Structure):
+    _fields_ = [("total_loss", C.c_double), ("min_lambda", C.c_double), ("max_lambda", C.c_double), ("peaks", C.c_int32),
+                ("peak_start", C.c_int32), ("peak_end", C.c_int32), ("selectable", C.c_int32), ("fp", C.c_int32),
+                ("fn", C.c_int32), ("possible_fp", C.c_int32), ("possible_fn", C.c_int32), ("errors", C.c_int32),
+                ("pad_", C.c_int32)]
+
+
+class PsdJointStats(C.Structure):
+    _fields_ = [("device_ms", C.c_double), ("kernel_ms", C.c_double), ("samples", C.c_int64), ("pair_sample_evals", C.c_int64),
+                ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64), ("n_problems", C.c_int32), ("n_waves", C.c_int32),
+                ("n_launches", C.c_int32), ("pad_", C.c_int32)]
+
+
 # every symbol include/peaksegdisk_b200.h declares (tests check the library exports all of them)
 C_ABI_SYMBOLS = [
     "psd_fpop_disk", "psd_fpop_disk_batch", "psd_status_message", "psd_last_error", "psd_plan_create",
@@ -95,6 +119,8 @@ C_ABI_SYMBOLS = [
     "psd_coverage_from_reads", "psd_coverage_n_rows", "psd_coverage_rows", "psd_coverage_get_stats", "psd_coverage_free",
     "psd_plan_set_labels", "psd_plan_label_errors", "psd_model_path", "psd_path_status", "psd_path_n_models",
     "psd_path_models", "psd_path_target", "psd_path_get_stats", "psd_path_free", "psd_features",
+    "psd_joint_models", "psd_joint_n_models", "psd_joint_model_table", "psd_joint_samples", "psd_joint_target",
+    "psd_joint_get_stats", "psd_joint_free",
     "_Z16PeakSegFPOP_diskPcS_S_",   # the reference's own C++-linkage entry (src/PeakSegFPOPLog.h:15)
 ]
 
@@ -178,6 +204,20 @@ def _load():
     lib.psd_features.restype = C.c_int
     lib.psd_features.argtypes = [C.c_int, C.c_int, C.POINTER(PsdRows), C.POINTER(PsdProblemFeatures),
                                  C.POINTER(PsdFeaturesStats)]
+    lib.psd_joint_models.restype = C.c_int
+    lib.psd_joint_models.argtypes = [C.c_int, C.c_int, C.POINTER(PsdJointProblem), C.POINTER(C.c_void_p)]
+    lib.psd_joint_n_models.restype = C.c_int
+    lib.psd_joint_n_models.argtypes = [C.c_void_p, C.c_int]
+    lib.psd_joint_model_table.restype = C.c_int
+    lib.psd_joint_model_table.argtypes = [C.c_void_p, C.c_int, C.POINTER(PsdJointModel)]
+    lib.psd_joint_samples.restype = C.c_int
+    lib.psd_joint_samples.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_uint8)]
+    lib.psd_joint_target.restype = C.c_int
+    lib.psd_joint_target.argtypes = [C.c_void_p, C.c_int, dp, dp, i32p]
+    lib.psd_joint_get_stats.restype = C.c_int
+    lib.psd_joint_get_stats.argtypes = [C.c_void_p, C.POINTER(PsdJointStats)]
+    lib.psd_joint_free.restype = None
+    lib.psd_joint_free.argtypes = [C.c_void_p]
     return lib
 
 

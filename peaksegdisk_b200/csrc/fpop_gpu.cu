@@ -9,6 +9,9 @@
 //   features_hist_kernel, features_select_kernel (x 4)
 //                          (psd_features only, not part of a plan) per-problem coverage statistics by
 //                          a weighted radix select over the rows (features_gpu.cuh).
+//   joint_flank_kernel, joint_flat_kernel, joint_pair_kernel<J>, joint_reduce_kernel
+//                          (psd_joint_models only, not part of a plan) exact joint single-peak models
+//                          of many samples (joint_gpu.cuh).
 //   fpop_dp_kernel<W,B>    persistent warps; each warp takes problems (longest first) from an atomic
 //                          queue and runs dp_run_queue() (fpop_warp.cuh): the whole DP of one
 //                          (bedGraph x penalty), piece lists in shared memory (moving to a per-warp
@@ -53,6 +56,7 @@ __device__ unsigned long long psd_blk_end[160];
 #endif
 __device__ const uint64_t d_exp_tab[256] = PSD_EXP_TAB_INIT;
 __device__ const uint64_t d_log_tab[256] = PSD_LOG_TAB_INIT;
+#include "joint_gpu.cuh"   // after d_log_tab: its kernels copy the table to shared memory
 
 static inline unsigned long long psd_ws_bytes(int cap, int ccap) { return cap > 0 ? PSD_WS_BYTES(cap, ccap) : PSD_WS_HDR; }
 
@@ -163,7 +167,7 @@ int psd_set_option_impl(const char* name, double value) {
   else if (n == "spill_mode") g_opt.spill_mode = (int)value;           // 0 DMA drain of an HBM ring (cudaMemcpyAsync on a side stream), 1 zero-copy stores
   else if (n == "ring_gb") g_opt.ring_gb = value;                      // HBM ring of the DMA drain (0 = automatic)
   else if (n == "devices") g_opt.devices = (int)value;                 // 1 current device only, k first k GPUs, <= 0 all
-  else if (n == "coverage_gb") g_opt.coverage_gb = value;              // psd_coverage_from_reads wave budget (0 = half of free HBM)
+  else if (n == "coverage_gb") g_opt.coverage_gb = value;              // psd_coverage_from_reads / psd_features / psd_joint_models wave budget (0 = half of free HBM)
   else return PSD_ERR_ARG;
   return 0;
 }
@@ -1774,6 +1778,191 @@ int psd_features_impl(int device, int n, const psd_rows* P, psd_problem_features
     }
   }
   if (stats) *stats = S;
+  return 0;
+}
+
+// ---- joint single-peak models (psd_joint_models, joint_gpu.cuh) -------------------------------------
+namespace {
+struct JointScratch {
+  unsigned char* d_arena = nullptr;
+  int64_t* p_pref = nullptr;   // prefix sums of a wave, pinned
+  cudaEvent_t ev[4]; bool ev_ok = false;
+  ~JointScratch() {
+    if (d_arena) cudaFree(d_arena);
+    if (p_pref) cudaFreeHost(p_pref);
+    if (ev_ok) for (auto& e : ev) cudaEventDestroy(e);
+  }
+};
+
+int joint_lanes(int S) { int j = 1; while (32 * j < S) j <<= 1; return j; }   // J: keys per lane
+
+// device bytes of a wave (the arena is carved in this order, see psd_joint_device)
+size_t joint_wave_bytes(int64_t n_probs, int64_t elems, int64_t tiles, int64_t chunks, int64_t cands, int64_t items) {
+  return cov_align(8 * elems) * 3 + cov_align(sizeof(JointProblem) * n_probs) + cov_align(8 * n_probs) + cov_align(4 * tiles) +
+         cov_align(sizeof(JointChunk) * chunks) + cov_align(8 * cands) + cov_align(4 * cands) + cov_align(sizeof(JointItem) * items) +
+         cov_align(8 * items) + cov_align(4 * items);
+}
+}  // namespace
+
+// Waves of consecutive problems that fit the "coverage_gb" budget: H2D of the prefix sums and the tables,
+// the flank, flat, pair (one launch per J present) and reduce kernels, D2H of one (loss, t) per (problem, k).
+int psd_joint_device(int device, const std::vector<JointDeviceProblem>& P, double* out_loss, int32_t* out_t, psd_joint_stats* S) {
+  const int n = (int)P.size();
+  if (n == 0) return 0;
+  int ndev = 0;
+  if (!cuda_ok(cudaGetDeviceCount(&ndev), "cudaGetDeviceCount")) return PSD_ERR_CUDA;
+  if (ndev == 0) { g_last_error = "no CUDA device"; return PSD_ERR_CUDA; }
+  if (device < 0) CK(cudaGetDevice(&device));
+  CK(cudaSetDevice(device));
+  cudaDeviceProp prop;
+  CK(cudaGetDeviceProperties(&prop, device));
+  if (prop.major < 10) { g_last_error = "peaksegdisk_b200 is built for sm_100a only"; return PSD_ERR_CUDA; }
+  // one chunk size for the call: about 64 chunks per warp slot of the device, at least 8 pairs
+  std::vector<int64_t> pairs(n), chunks(n), tiles(n), elems(n);
+  int64_t all_pairs = 0;
+  for (int k = 0; k < n; k++) {
+    const int64_t N = P[k].N;
+    pairs[k] = (N - 1) * (N - 2) / 2;
+    all_pairs += pairs[k];
+  }
+  const int64_t target = (int64_t)prop.multiProcessorCount * 64 * 64;
+  const int64_t cp = std::max<int64_t>(8, (all_pairs + target - 1) / target);
+  for (int k = 0; k < n; k++) {
+    chunks[k] = (pairs[k] + cp - 1) / cp;
+    elems[k] = (int64_t)(P[k].N + 1) * P[k].S;
+    tiles[k] = (elems[k] + PSD_JOINT_FLANK_TILE - 1) / PSD_JOINT_FLANK_TILE;
+  }
+  JointScratch X;
+  for (auto& e : X.ev) CK(cudaEventCreate(&e));
+  X.ev_ok = true;
+  size_t free_b = 0, total_b = 0;
+  CK(cudaMemGetInfo(&free_b, &total_b));
+  const double gb = current_options().coverage_gb;
+  const size_t budget = gb > 0 ? (size_t)(gb * (double)(1ull << 30)) : free_b / 2;
+  std::vector<std::pair<int, int>> waves;   // [first problem, end problem)
+  size_t arena = 0, max_elems = 0;
+  for (int k0 = 0; k0 < n;) {
+    int k1 = k0;
+    int64_t e = 0, t = 0, c = 0, cd = 0, it = 0;
+    size_t bytes = 0;
+    for (; k1 < n; k1++) {
+      const size_t b = joint_wave_bytes(k1 - k0 + 1, e + elems[k1], t + tiles[k1], c + chunks[k1], cd + chunks[k1] * P[k1].S, it + P[k1].S);
+      if (k1 > k0 && b > budget) break;
+      e += elems[k1]; t += tiles[k1]; c += chunks[k1]; cd += chunks[k1] * P[k1].S; it += P[k1].S; bytes = b;
+    }
+    waves.push_back({k0, k1});
+    arena = std::max(arena, bytes); max_elems = std::max(max_elems, (size_t)e);
+    k0 = k1;
+  }
+  CK(cudaMalloc(&X.d_arena, arena));
+  CK(cudaMallocHost(&X.p_pref, 8 * max_elems));
+  const cudaStream_t st = 0;
+  for (const auto& w : waves) {
+    const int np = w.second - w.first;
+    std::vector<JointProblem> probs(np);
+    std::vector<int> tile_prob;
+    std::vector<JointItem> items;
+    std::vector<JointChunk> chunk_tab;
+    std::vector<std::pair<int, int>> j_range;   // per J present: [first chunk, end chunk)
+    int64_t e = 0, cd = 0;
+    for (int j = 0; j < np; j++) {
+      const JointDeviceProblem& D = P[w.first + j];
+      JointProblem& q = probs[j];
+      q.grid_off = e; q.cand_off = cd; q.S = D.S; q.N = D.N; q.bin = D.bin; q.len = D.len;
+      q.n_chunks = (int)chunks[w.first + j]; q.tile0 = (int)tile_prob.size();
+      tile_prob.insert(tile_prob.end(), (size_t)tiles[w.first + j], j);
+      for (int k = 1; k <= D.S; k++) items.push_back({j, k});
+      memcpy(X.p_pref + e, D.pref, 8 * (size_t)elems[w.first + j]);
+      e += elems[w.first + j]; cd += (int64_t)q.n_chunks * D.S;
+    }
+    for (int J = 1; J <= 8; J <<= 1) {   // the chunks grouped by J, one pair-kernel launch per group
+      const int c0 = (int)chunk_tab.size();
+      for (int j = 0; j < np; j++) {
+        JointProblem& q = probs[j];
+        if (joint_lanes(q.S) != J) continue;
+        q.chunk0 = (int)chunk_tab.size();
+        int a = 1, b = 2;
+        for (int64_t t0 = 0; t0 < pairs[w.first + j]; t0 += cp) {
+          const int cnt = (int)std::min<int64_t>(cp, pairs[w.first + j] - t0);
+          chunk_tab.push_back({j, a, b, (int)t0, cnt});
+          for (int r = cnt; r > 0;) {   // advance (a, b) by cnt pairs
+            const int left = q.N - b;   // pairs left in row a, b included
+            if (r < left) { b += r; r = 0; } else { r -= left; a++; b = a + 1; }
+          }
+        }
+      }
+      if ((int)chunk_tab.size() > c0) j_range.push_back({c0, (int)chunk_tab.size()});
+      else j_range.push_back({c0, c0});
+    }
+    const int n_tiles = (int)tile_prob.size(), n_chunks = (int)chunk_tab.size(), n_items = (int)items.size();
+    unsigned char* ar = X.d_arena;
+    auto carve = [&](size_t b) { unsigned char* r = ar; ar += cov_align(b); return r; };
+    JointParams K;
+    memset(&K, 0, sizeof K);
+    long long* d_pref = (long long*)carve(8 * e);
+    K.pref = d_pref;
+    K.lleft = (double*)carve(8 * e);
+    K.lright = (double*)carve(8 * e);
+    JointProblem* d_probs = (JointProblem*)carve(sizeof(JointProblem) * np);
+    K.probs = d_probs;
+    K.flat = (double*)carve(8 * np);
+    int* d_tile = (int*)carve(4 * (size_t)n_tiles);
+    K.tile_prob = d_tile; K.n_tiles = n_tiles; K.n_probs = np;
+    JointChunk* d_chunks = (JointChunk*)carve(sizeof(JointChunk) * n_chunks);
+    K.chunks = d_chunks;
+    K.cand_loss = (double*)carve(8 * cd);
+    K.cand_t = (int*)carve(4 * cd);
+    JointItem* d_items = (JointItem*)carve(sizeof(JointItem) * n_items);
+    K.items = d_items; K.n_items = n_items;
+    K.out_loss = (double*)carve(8 * (size_t)n_items);
+    K.out_t = (int*)carve(4 * (size_t)n_items);
+    CK(cudaEventRecord(X.ev[0], st));
+    CK(cudaMemcpyAsync(d_pref, X.p_pref, 8 * e, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_probs, probs.data(), sizeof(JointProblem) * np, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_tile, tile_prob.data(), 4 * (size_t)n_tiles, cudaMemcpyHostToDevice, st));
+    if (n_chunks) CK(cudaMemcpyAsync(d_chunks, chunk_tab.data(), sizeof(JointChunk) * n_chunks, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_items, items.data(), sizeof(JointItem) * n_items, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(X.ev[1], st));
+    joint_flank_kernel<<<n_tiles, 256, 0, st>>>(K);
+    CK(cudaGetLastError());
+    joint_flat_kernel<<<(np + 127) / 128, 128, 0, st>>>(K);
+    CK(cudaGetLastError());
+    S->n_launches += 3;
+    for (int g = 0; g < 4; g++) {
+      K.chunk_begin = j_range[g].first; K.chunk_end = j_range[g].second;
+      const int nc = K.chunk_end - K.chunk_begin;
+      if (nc == 0) continue;
+      const int blocks = (nc + PSD_JOINT_WARPS - 1) / PSD_JOINT_WARPS;
+      if (g == 0) joint_pair_kernel<1><<<blocks, PSD_JOINT_WARPS * 32, 0, st>>>(K);
+      else if (g == 1) joint_pair_kernel<2><<<blocks, PSD_JOINT_WARPS * 32, 0, st>>>(K);
+      else if (g == 2) joint_pair_kernel<4><<<blocks, PSD_JOINT_WARPS * 32, 0, st>>>(K);
+      else joint_pair_kernel<8><<<blocks, PSD_JOINT_WARPS * 32, 0, st>>>(K);
+      CK(cudaGetLastError());
+      S->n_launches++;
+    }
+    joint_reduce_kernel<<<(n_items + 7) / 8, 256, 0, st>>>(K);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(X.ev[2], st));
+    std::vector<double> loss(n_items);
+    std::vector<int> tt(n_items);
+    CK(cudaMemcpyAsync(loss.data(), K.out_loss, 8 * (size_t)n_items, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(tt.data(), K.out_t, 4 * (size_t)n_items, cudaMemcpyDeviceToHost, st));
+    CK(cudaEventRecord(X.ev[3], st));
+    CK(cudaStreamSynchronize(st));
+    float t03 = 0, t12 = 0;
+    cudaEventElapsedTime(&t03, X.ev[0], X.ev[3]); cudaEventElapsedTime(&t12, X.ev[1], X.ev[2]);
+    S->device_ms += t03; S->kernel_ms += t12;
+    S->n_waves++;
+    S->h2d_bytes += 8 * e + (int64_t)sizeof(JointProblem) * np + 4 * (int64_t)n_tiles + (int64_t)sizeof(JointChunk) * n_chunks +
+                    (int64_t)sizeof(JointItem) * n_items;
+    S->d2h_bytes += 12 * (int64_t)n_items;
+    int o = 0;
+    for (int j = 0; j < np; j++) {
+      const JointDeviceProblem& D = P[w.first + j];
+      S->pair_sample_evals += pairs[w.first + j] * D.S;
+      for (int k = 0; k < D.S; k++, o++) { out_loss[D.out_off + k] = loss[o]; out_t[D.out_off + k] = tt[o]; }
+    }
+  }
   return 0;
 }
 

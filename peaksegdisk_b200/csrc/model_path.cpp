@@ -49,25 +49,6 @@ struct Problem {
 
 struct Job { int prob; int pair; double penalty; };   // pair -1: a round-1 solve
 
-// Target interval: the widest run (in log penalty) of consecutive models with the fewest errors; a run
-// that reaches 0 or infinity is infinitely wide; ties go to the smaller min_lambda.
-void target_interval(const std::vector<psd_path_model>& m, double* lo, double* hi, int* errors) {
-  int best = m[0].errors;
-  for (const auto& x : m) best = std::min(best, x.errors);
-  double best_w = -1, best_lo = NAN, best_hi = NAN;
-  for (size_t a = 0; a < m.size();) {
-    if (m[a].errors != best) { a++; continue; }
-    size_t b = a;
-    while (b + 1 < m.size() && m[b + 1].errors == best) b++;
-    // models are sorted by peaks ascending, so lambda decreases from a to b
-    const double r_hi = m[a].max_lambda, r_lo = m[b].min_lambda;
-    const double w = (r_lo == 0 || std::isinf(r_hi)) ? INFINITY : std::log(r_hi) - std::log(r_lo);
-    if (best_w < 0 || w > best_w || (w == best_w && r_lo < best_lo)) { best_w = w; best_lo = r_lo; best_hi = r_hi; }
-    a = b + 1;
-  }
-  *lo = best_lo; *hi = best_hi; *errors = best;
-}
-
 }  // namespace
 
 static int model_path_impl(int device, int n, const psd_path_problem* P, double pen_min, double pen_max, psd_path** out) {

@@ -128,3 +128,16 @@ HostProblem make_row_problem(int64_t n_rows, const int32_t* chromStart, const in
 int make_label_set(const HostProblem& h, int64_t n, const int32_t* start, const int32_t* end, const int32_t* kind,
                    std::shared_ptr<const LabelSet>* out, std::string* why);
 const std::string& psd_get_last_error();
+// the target interval of psd_model_path and psd_joint_models (host_api.cpp): models sorted by peaks ascending
+void target_interval(const std::vector<psd_path_model>& m, double* lo, double* hi, int* errors);
+
+// joint.cpp -> fpop_gpu.cu: one problem of psd_joint_models as the device sees it (problems with N >= 3)
+struct JointDeviceProblem {
+  int S, N, bin, len;      // samples, bins, bin width, region length
+  const int64_t* pref;     // C_s(0, i), (N + 1) * S entries, [grid index][sample]
+  int64_t out_off;         // its S results (k = 1..S) in out_loss / out_t
+};
+// For every problem and k = 1..S the minimum of loss_k over all peaks (joint_gpu.cuh): out_loss, and out_t the
+// flattened pair index (-1: no pair has k feasible samples).  Adds device time, waves, launches, copies and
+// pair x sample evaluations to *stats.
+int psd_joint_device(int device, const std::vector<JointDeviceProblem>& probs, double* out_loss, int32_t* out_t, psd_joint_stats* stats);

@@ -377,3 +377,96 @@ def model_path_batch(problems, labels=None, pen_min=0.0, pen_max=math.inf, devic
         return paths, {name: getattr(st, name) for name, _ in st._fields_}
     finally:
         _lib.lib.psd_path_free(h)
+
+
+JOINT_COLUMNS = ["peaks", "total.loss", "peakStart", "peakEnd", "selectable", "min.lambda", "max.lambda",
+                 "min.log.lambda", "max.log.lambda"]
+
+
+def joint_models_batch(problems, bin_bases=1, labels=None, device=-1):
+    """Exact joint single-peak models (the model of PeakSegJoint: one peak shared by position, per-sample
+    means, the number of peaked samples as the complexity) of many regions in ONE psd_joint_models call.
+    problems: per region, a list with one (chromStart, chromEnd, coverage) per sample; the region is sample 0's
+    [first chromStart, last chromEnd), and every sample's rows must tile it.  bin_bases: the grid's bin width
+    (peak ends are on bin boundaries).  labels: None or, per problem, a list with one label DataFrame (or None)
+    per sample; label errors are summed over samples.
+
+    Returns (results, stats).  results[i] is {"models": DataFrame, "in_peak": bool array (models x samples),
+    "target": (min.lambda, max.lambda, errors) or None}; the models, one per k that has one (k ascending), have
+    the columns peaks (k), total.loss, peakStart, peakEnd (-1 for k = 0), selectable, min.lambda, max.lambda,
+    min.log.lambda, max.log.lambda (NaN when not selectable) and, with labels, fp, fn, possible.fp, possible.fn
+    and errors.  stats is the call's psd_joint_stats as a dict."""
+    import pandas as pd
+    problems = [list(p) for p in problems]
+    if labels is None:
+        labels = [None] * len(problems)
+    labels = list(labels)
+    if len(labels) != len(problems):
+        raise ValueError("labels needs one entry (a list per sample, or None) per problem")
+    arr = (_lib.PsdJointProblem * max(1, len(problems)))()
+    keep = []   # the int32 copies and sample arrays must outlive the call
+    p32 = C.POINTER(C.c_int32)
+    has_labels = []
+    for i, (samples, lab) in enumerate(zip(problems, labels)):
+        if lab is not None:
+            lab = list(lab)
+            if len(lab) != len(samples):
+                raise ValueError("problem %d: labels needs one entry (a DataFrame or None) per sample" % i)
+        sa = (_lib.PsdJointSample * max(1, len(samples)))()
+        keep.append(sa)
+        for j, (s, e, c) in enumerate(samples):
+            s, sp = _i32(s)
+            e, ep = _i32(e)
+            c, cp = _i32(c)
+            if not (len(s) == len(e) == len(c)):
+                raise ValueError("problem %d sample %d: chromStart, chromEnd and coverage must have the same length" % (i, j))
+            keep += [s, e, c]
+            sa[j].n_rows = len(c); sa[j].chromStart = sp; sa[j].chromEnd = ep; sa[j].coverage = cp
+            if lab is not None and lab[j] is not None:
+                ls, le, lk = label_arrays(lab[j])
+                keep += [ls, le, lk]
+                sa[j].n_labels = len(lk)
+                sa[j].label_start = ls.ctypes.data_as(p32); sa[j].label_end = le.ctypes.data_as(p32)
+                sa[j].label_kind = lk.ctypes.data_as(p32)
+        s0 = samples[0] if samples else None
+        if s0 is not None and len(s0[0]):
+            arr[i].region_start = int(s0[0][0]); arr[i].region_end = int(s0[1][-1])
+        arr[i].bin_bases = int(bin_bases); arr[i].n_samples = len(samples); arr[i].samples = sa
+        has_labels.append(lab is not None and any(x is not None for x in lab))
+    h = C.c_void_p()
+    rc = _lib.lib.psd_joint_models(int(device), len(problems), arr, C.byref(h))
+    if rc == 111:
+        raise ValueError("peaksegdisk_b200: " + _lib.lib.psd_last_error().decode())
+    if rc:
+        raise RuntimeError("peaksegdisk_b200: " + _lib.status_text(rc))
+    try:
+        out = []
+        for i in range(len(problems)):
+            n = _lib.lib.psd_joint_n_models(h, i)
+            m = (_lib.PsdJointModel * n)()
+            _lib.lib.psd_joint_model_table(h, i, m)
+            a = np.ctypeslib.as_array(m)
+            lo, hi = a["min_lambda"].copy(), a["max_lambda"].copy()
+            with np.errstate(divide="ignore"):
+                cols = {"peaks": a["peaks"].astype(np.int64), "total.loss": a["total_loss"].copy(),
+                        "peakStart": a["peak_start"].astype(np.int64), "peakEnd": a["peak_end"].astype(np.int64),
+                        "selectable": a["selectable"] != 0, "min.lambda": lo, "max.lambda": hi,
+                        "min.log.lambda": np.log(lo), "max.log.lambda": np.log(hi)}
+            S = len(problems[i])
+            flags = np.zeros((n, S), np.uint8)
+            for r in range(n):
+                _lib.lib.psd_joint_samples(h, i, int(a["peaks"][r]), flags[r].ctypes.data_as(C.POINTER(C.c_uint8)))
+            target = None
+            if has_labels[i]:
+                for col, f in zip(PATH_ERROR_COLUMNS, ["fp", "fn", "possible_fp", "possible_fn", "errors"]):
+                    cols[col] = a[f].astype(np.int64)
+                tlo, thi, terr = C.c_double(), C.c_double(), C.c_int32()
+                _lib.lib.psd_joint_target(h, i, C.byref(tlo), C.byref(thi), C.byref(terr))
+                if terr.value >= 0:
+                    target = (tlo.value, thi.value, terr.value)
+            out.append({"models": pd.DataFrame(cols), "in_peak": flags.astype(bool), "target": target})
+        st = _lib.PsdJointStats()
+        _lib.lib.psd_joint_get_stats(h, C.byref(st))
+        return out, {name: getattr(st, name) for name, _ in st._fields_}
+    finally:
+        _lib.lib.psd_joint_free(h)
